@@ -25,6 +25,8 @@ for a circuit of the shape named in `config.workload`, on synthetic seeded colum
                 inside the library on the launching stream.
   * `cpu_baseline` / `--impl reference`: the CPU restatement of halo2's Rayon algorithms (oracle/, "port") running the WHOLE
                 trace for real on the box's host cores (a persistent thread pool, every op instance executed, nothing extrapolated).
+--dump-outputs DIR: after the timed steps, DIR/<name>.npy holds what the last timed step computed (see dump_outputs); the inputs
+are seeded, so two builds run with the same arguments can be compared output for output.
 --simulate-rank-of N: ONE GPU executes rank 0's share of an N-way run (same deal, same kernels, exchanges skipped) so that a rank's
 per-step kernel list can be profiled without N GPUs; the line is marked SIMULATED and is not a bench value.
 N > 1 (torchrun): independent columns are dealt round-robin to ranks (strong scaling, no data-path collective inside an
@@ -111,6 +113,33 @@ def gate_program(m):
         a, b, c = ev.Query(t), ev.Query((t + 1) % m, 1), ev.Query((t + 2) % m, -1)
         value = value * y + (a * b + c * a - b)
     return ev.QuotientProgram(value)
+
+
+DUMP_QUOTIENT_ROWS = 1 << 19      # 32 MB of quotient digits; with the rest, a dump stays under 64 MB at every k
+
+
+def wire_digits(a):
+    """uint64 wire limbs [..., L] -> float32 [..., 4L]: the same bits as little-endian 16-bit digits, exact in float32, so a
+    difference of one in any limb survives a float comparison."""
+    a = np.ascontiguousarray(a).view(np.uint64)
+    return a.view("<u2").reshape(a.shape[:-1] + (4 * a.shape[-1],)).astype(np.float32)
+
+
+def dump_outputs(out_dir, commits_xyzz, evals, h):
+    """Writes one step's results in the library's wire format (Montgomery limbs) through wire_digits: the commitments (normalised
+    Jacobian), the evaluations, and the quotient's coefficients (all of them, or a seeded sample of DUMP_QUOTIENT_ROWS rows, whose
+    row numbers go to quotient_rows.npy)."""
+    import torch
+    from ezkl_b200 import device as dev
+    os.makedirs(out_dir, exist_ok=True)
+    rows = h.shape[0]
+    pick = np.arange(rows) if rows <= DUMP_QUOTIENT_ROWS else np.sort(np.random.default_rng(0xD0).choice(rows, DUMP_QUOTIENT_ROWS, replace=False))
+    out = {"commitments": wire_digits(dev.normalize(commits_xyzz)),
+           "evaluations": wire_digits(dev.to_host(torch.cat(evals))),
+           "quotient": wire_digits(dev.to_host(h[torch.from_numpy(pick).to(h.device)])),
+           "quotient_rows": pick.astype(np.float64)}
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler(threading.Thread):
@@ -376,6 +405,7 @@ def run_b200(args):
         _g += _count
 
     evals = []
+    quotient = {}
     npolys_total = tr["advice"] + tr["fixed"] + tr["perm_cols"] + tr["perm_z"] + 2 * tr["lookups"] + 1 + tr["quotient_pieces"]
     lin_scalars = np.ascontiguousarray(np.tile(xs, (npolys_total // ncols + 1, 1))[:npolys_total])
 
@@ -426,7 +456,7 @@ def run_b200(args):
                     if fut is not None:
                         fut.result()                  # the side thread has ENQUEUED everything (its done event is recorded); no device sync
                         fut = None
-                    quotient_stage(lambda j: cols_[j % ncols], None, early=two)
+                    quotient_stage(lambda j: cols_[j % ncols], lambda h: quotient.update(h=h), early=two)
                 elif kind == "eval":
                     evals.append(dev.eval_batch(v, xs[:b]))
                 elif kind == "lincomb":
@@ -625,13 +655,15 @@ def run_b200(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        step_device()
+        pts = step_device()
     e1.record()
     issue_ms = (time.time() - t_reg0) * 1e3 / args.steps     # host time to ENQUEUE a step (close to ms_per_step means the host issue rate is the limiter)
     barrier()
     sampler.mark(t_reg0, time.time())
     launches = nat.launch_count() - l0
     ms_dev = max_over_ranks(e0.elapsed_time(e1)) / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, pts, evals, quotient["h"])
     # ---- same steps again with per-kernel-class CUDA events (roofline leg; not part of `value`)
     nat.check(L.b200_profile_enable(1))
     coll["on"] = True
@@ -908,7 +940,11 @@ def main():
     ap.add_argument("--profile-one-step", action="store_true", help="setup + one device step only (for ncu launch lists)")
     ap.add_argument("--no-overlap", action="store_true", help="single-stream schedule (trace order), for A/B against the two-stream schedule")
     ap.add_argument("--simulate-rank-of", type=int, default=0, help="profiling aid: run rank 0's share of an N-way run on ONE GPU (collectives skipped); the line is marked SIMULATED")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy (float32 digits of the wire limbs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
     if args.impl == "reference":

@@ -1,19 +1,25 @@
 #!/usr/bin/env python
 """Regenerates tests/golden/* from the reference's own checked-in fixtures.
 
-Run in the build container only (reads /root/reference, which does not exist on the GPU box):
-    python tests/golden/make_golden.py
+Needs a checkout of zkonduit/ezkl; the tests read only what this writes:
+    python tests/golden/make_golden.py <ezkl checkout>/tests/assets
 
 Inputs (reference fixtures, SURVEY.md Appendix B):
-  /root/reference/tests/assets/kzg     ParamsKZG::write output for k=6 (what src/pfsys/srs.rs:40-47 reads)
-  /root/reference/tests/assets/pk.key  ProvingKey::write (RawBytes), read by src/pfsys/mod.rs:615
+  kzg         ParamsKZG::write output for k=6 (what src/pfsys/srs.rs:40-47 reads)
+  pk.key      ProvingKey::write (RawBytes), read by src/pfsys/mod.rs:615
+  proof.json  a proof of the k=6 fixture circuit made by the Rust prover
 
 Outputs:
   tests/golden/kzg_k6.srs           the 8452-byte SRS data fixture, verbatim (data, not source)
   tests/golden/pk_k6_subset.npz     a few columns of the proving key:
       fixed_values/fixed_polys/fixed_cosets[c]  c in FIXED_COLS, perm_{values,polys,cosets}[0],
       l0, l_last, l_active_row   -- all as uint64[.,4] little-endian Montgomery limbs (the wire form)
-  tests/golden/manifest.json        sizes + sha256 of both, and the relations verified while generating
+  tests/golden/pk_k6_vk.bin         the verifying-key bytes that open pk.key, verbatim
+  tests/golden/pk_k6_values.npy     every fixed column's values, then every permutation column's, uint64[38 + 32, 64, 4];
+      with the above, enough to rebuild pk.key byte for byte (tests/helpers.py write_reference_pk; the polys and
+      cosets in it are derived from these values)
+  tests/golden/reference_proof_k6.bin  the proof bytes of proof.json
+  tests/golden/manifest.json        sizes + sha256 of the outputs and of pk.key, and the relations verified while generating
 
 Known-answer content these fixtures give the hot path:
   * 64 MSM known answers:  g_lagrange[j] = n^-1 * sum_i omega^(-ij) * g[i]     (pins MSM, omega, G1 add)
@@ -32,7 +38,6 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "..", ".."))
 from oracle import pyref as ref  # noqa: E402
 
-ASSETS = "/root/reference/tests/assets"
 FIXED_COLS = [0, 1, 5, 37]
 
 
@@ -77,6 +82,7 @@ def parse_pk(d: bytes):
     off += 64 * nperm
     nsel = 80
     off += nsel * (n // 8)
+    vk = d[:off]
     l0, off = read_poly(d, off)
     l_last, off = read_poly(d, off)
     l_active, off = read_poly(d, off)
@@ -87,7 +93,7 @@ def parse_pk(d: bytes):
     perm_polys, off = read_slice(d, off)
     perm_cosets, off = read_slice(d, off)
     assert off == len(d), (off, len(d))
-    return dict(k=k, l0=l0, l_last=l_last, l_active_row=l_active, fixed_values=fixed_values,
+    return dict(k=k, vk=vk, l0=l0, l_last=l_last, l_active_row=l_active, fixed_values=fixed_values,
                 fixed_polys=fixed_polys, fixed_cosets=fixed_cosets, perms=perms, perm_polys=perm_polys,
                 perm_cosets=perm_cosets)
 
@@ -100,9 +106,18 @@ def frs(b: bytes):
     return [ref.fr_from_wire(b[i:i + 32]) for i in range(0, len(b), 32)]
 
 
-def main():
+def save_npz_if_changed(path, arrays):
+    """np.savez stamps the time into the archive: keep the committed file when its arrays are already these."""
+    if os.path.exists(path):
+        old = np.load(path)
+        if set(old.files) == set(arrays) and all(np.array_equal(old[name], a) for name, a in arrays.items()):
+            return
+    np.savez_compressed(path, **arrays)
+
+
+def main(assets):
     checks = []
-    srs = open(os.path.join(ASSETS, "kzg"), "rb").read()
+    srs = open(os.path.join(assets, "kzg"), "rb").read()
     k, g, gl = parse_srs(srs)
     n = 1 << k
     gp = [ref.g1_from_wire(x) for x in g]
@@ -119,7 +134,8 @@ def main():
     with open(os.path.join(HERE, "kzg_k6.srs"), "wb") as f:
         f.write(srs)
 
-    pk = parse_pk(open(os.path.join(ASSETS, "pk.key"), "rb").read())
+    pk_bytes = open(os.path.join(assets, "pk.key"), "rb").read()
+    pk = parse_pk(pk_bytes)
     assert pk["k"] == 6
     ext_k = 9
     out = {}
@@ -146,15 +162,27 @@ def main():
     assert ref.coeff_to_extended(llc, 6, ext_k) == frs(pk["l_last"])
     checks.append("pk: l0 == coset-extended L_0, l_last == coset-extended L_{n-6}")
     out["l0"], out["l_last"], out["l_active_row"] = limbs(pk["l0"]), limbs(pk["l_last"]), limbs(pk["l_active_row"])
-    np.savez_compressed(os.path.join(HERE, "pk_k6_subset.npz"), **out)
+    save_npz_if_changed(os.path.join(HERE, "pk_k6_subset.npz"), out)
+    with open(os.path.join(HERE, "pk_k6_vk.bin"), "wb") as f:
+        f.write(pk["vk"])
+    np.save(os.path.join(HERE, "pk_k6_values.npy"), np.stack([limbs(v) for v in pk["fixed_values"] + pk["perms"]]))
 
-    man = {"source": "zkonduit/ezkl tests/assets/{kzg,pk.key}", "k": 6, "ext_k": ext_k, "checks": checks}
-    for fn in ("kzg_k6.srs", "pk_k6_subset.npz"):
+    proof = bytes(json.load(open(os.path.join(assets, "proof.json")))["proof"])
+    assert len(proof) == 114 * 64 + 231 * 32 + 2 * 64
+    checks.append("proof: 114 commitments, 231 evaluations, 2 SHPLONK points")
+    with open(os.path.join(HERE, "reference_proof_k6.bin"), "wb") as f:
+        f.write(proof)
+
+    man = {"source": "zkonduit/ezkl tests/assets/{kzg,pk.key,proof.json}", "k": 6, "ext_k": ext_k, "checks": checks}
+    for fn in ("kzg_k6.srs", "pk_k6_subset.npz", "pk_k6_vk.bin", "pk_k6_values.npy", "reference_proof_k6.bin"):
         b = open(os.path.join(HERE, fn), "rb").read()
         man[fn] = {"bytes": len(b), "sha256": hashlib.sha256(b).hexdigest()}
+    man["pk.key"] = {"bytes": len(pk_bytes), "sha256": hashlib.sha256(pk_bytes).hexdigest()}
     json.dump(man, open(os.path.join(HERE, "manifest.json"), "w"), indent=1)
     print("\n".join(checks))
 
 
 if __name__ == "__main__":
-    main()
+    if len(sys.argv) != 2:
+        raise SystemExit("usage: python tests/golden/make_golden.py <ezkl checkout>/tests/assets")
+    main(sys.argv[1])

@@ -63,3 +63,32 @@ def load_srs_fixture():
 
 def load_pk_fixture():
     return dict(np.load(os.path.join(GOLDEN, "pk_k6_subset.npz")))
+
+
+def write_reference_pk(path):
+    """Rebuilds the reference's k = 6 pk.key (ProvingKey::write, RawBytes) at `path` from tests/golden: the verifying-key bytes,
+    l0 / l_last / l_active_row and the Lagrange values of the 38 fixed and 32 permutation columns are stored; their coefficient
+    and extended-coset forms are derived with the CPU oracle.  The result must hash to the sha256 the manifest recorded for pk.key."""
+    import hashlib
+    import json
+    from oracle import oracle as orc
+    k, ext_k, n_fixed = 6, 9, 38
+    values = np.load(os.path.join(GOLDEN, "pk_k6_values.npy"))
+    polys = [orc.lagrange_to_coeff(v, k) for v in values]
+    cosets = [orc.coeff_to_extended(p, ext_k) for p in polys]
+    sub = load_pk_fixture()
+
+    def poly(a):
+        return struct.pack(">I", a.shape[0]) + np.ascontiguousarray(a, dtype="<u8").tobytes()
+
+    def slice_(arrs):
+        return struct.pack(">I", len(arrs)) + struct.pack(">%dI" % len(arrs), *[a.shape[0] for a in arrs]) + b"".join(poly(a) for a in arrs)
+
+    parts = [open(os.path.join(GOLDEN, "pk_k6_vk.bin"), "rb").read(), poly(sub["l0"]), poly(sub["l_last"]), poly(sub["l_active_row"])]
+    for lo, hi in ((0, n_fixed), (n_fixed, len(values))):
+        parts += [slice_(list(values[lo:hi])), slice_(polys[lo:hi]), slice_(cosets[lo:hi])]
+    data = b"".join(parts)
+    expected = json.load(open(os.path.join(GOLDEN, "manifest.json")))["pk.key"]
+    assert len(data) == expected["bytes"] and hashlib.sha256(data).hexdigest() == expected["sha256"], "rebuilt pk.key differs from the reference's"
+    with open(path, "wb") as f:
+        f.write(data)

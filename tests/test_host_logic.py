@@ -118,11 +118,10 @@ def test_signed_window_recoding(c):
         assert all(-(1 << (c - 1)) <= int(d) <= (1 << (c - 1)) for d in out[i])
 
 
-def test_proving_key_reader_on_reference_fixture():
-    """ProvingKey::read mirror against the reference's own tests/assets/pk.key (present in the build container only)."""
-    path = "/root/reference/tests/assets/pk.key"
-    if not os.path.exists(path):
-        pytest.skip("reference checkout not present (GPU box)")
+def test_proving_key_reader_on_reference_fixture(tmp_path):
+    """ProvingKey::read mirror against the reference's own tests/assets/pk.key, rebuilt byte for byte from tests/golden."""
+    path = str(tmp_path / "pk.key")
+    H.write_reference_pk(path)
     from ezkl_b200 import halo2 as h2
     pk = h2.ProvingKey.read(path, num_permutation_columns=32, num_selectors=80)
     g = H.load_pk_fixture()
@@ -151,6 +150,45 @@ def test_bench_reference_arm_prints_contract_json():
         assert key in line, key
     assert line["impl"] == "reference" and line["higher_is_better"] is False and line["cpu_baseline"]["kind"] == "port"
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and "workload" in line["config"]
+
+
+def test_bench_output_digits_are_exact():
+    """bench.py --dump-outputs writes wire limbs as float32 16-bit digits: every bit must come back."""
+    import sys
+    sys.path.insert(0, ROOT)
+    import bench
+    a = np.random.default_rng(3).integers(0, 1 << 63, size=(50, 4), dtype=np.uint64) * np.uint64(2) + np.uint64(1)
+    a[0], a[1] = 0, np.uint64(0xFFFFFFFFFFFFFFFF)
+    d = bench.wire_digits(a)
+    assert d.dtype == np.float32 and d.shape == (50, 16) and d.max() <= 0xFFFF
+    back = np.ascontiguousarray(d.astype(np.uint16)).view(np.uint64)
+    assert np.array_equal(back, a)
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_are_reproducible(tmp_path):
+    """Two bench runs with different --steps dump the same outputs (seeded inputs, every step recomputes them); the line reports
+    the steps that were asked for, and the dump has the trace's shapes, in float32 / float64, under 64 MB."""
+    import json
+    import subprocess
+    import sys
+    sys.path.insert(0, ROOT)
+    import bench
+    dumps = {}
+    for steps in (2, 1):
+        d = tmp_path / ("steps%d" % steps)
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--k", "9", "--steps", str(steps), "--warmup", "0", "--no-cpu-baseline",
+                            "--dump-outputs", str(d)], capture_output=True, text=True, timeout=900)
+        assert r.returncode == 0, r.stderr[-3000:]
+        assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == steps
+        dumps[steps] = {f: np.load(d / f) for f in sorted(os.listdir(d))}
+    tr = bench.TRACES[bench.CONFIG_FOR_K[9]]
+    n_commits = sum(c for kind, c in bench.trace_ops(tr) if kind.startswith("msm"))
+    got = dumps[1]
+    assert got["commitments.npy"].shape == (n_commits, 48) and got["evaluations.npy"].shape == (tr["evals"], 16)
+    assert got["quotient.npy"].shape == (tr["quotient_pieces"] << 9, 16)
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values()) and sum(a.nbytes for a in got.values()) <= 64 << 20
+    assert dumps[2].keys() == got.keys() and all(np.array_equal(dumps[2][f], got[f]) for f in got)
 
 
 def test_fp64_pipe_multiplier_vs_bigint():

@@ -1,7 +1,6 @@
 """create_proof mirror (ezkl_b200/prover.py) + EvmTranscript (ezkl_b200/transcript.py): Keccak known answers, the rng, the proof
 encoding against the reference's own fixture, and a full prove -> verify round trip on the ezkl-shaped constraint system."""
 import hashlib
-import json
 import os
 import random
 
@@ -71,12 +70,10 @@ def test_transcript_rules():
 
 
 def test_reference_proof_fixture_parses_with_the_read_transcript():
-    """The reference's own proof fixture (/root/reference/tests/assets/proof.json, made by the Rust prover): 114 commitments,
-    231 evaluations, 2 SHPLONK points — every point must pass the on-curve check of EvmTranscriptRead, every scalar must be canonical."""
-    path = "/root/reference/tests/assets/proof.json"
-    if not os.path.exists(path):
-        pytest.skip("reference checkout not present (GPU box)")
-    proof = bytes(json.load(open(path))["proof"])
+    """The reference's own proof fixture (tests/assets/proof.json, made by the Rust prover; its proof bytes are
+    tests/golden/reference_proof_k6.bin): 114 commitments, 231 evaluations, 2 SHPLONK points — every point must pass the on-curve
+    check of EvmTranscriptRead, every scalar must be canonical."""
+    proof = open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_proof_k6.bin"), "rb").read()
     rd = ts.EvmTranscriptRead(proof)
     assert len(proof) == 114 * 64 + 231 * 32 + 2 * 64
     pts = [rd.read_ec_point() for _ in range(114)]
