@@ -92,6 +92,20 @@ struct Ctx {
 static std::vector<Ctx*> g_ctxs;
 static std::atomic<int> g_nctx{0};
 
+// restores the calling thread's current device on every exit of a scope that switches devices with cudaSetDevice
+struct CurrentDevice {
+    int prev = 0;
+    CurrentDevice() { cudaGetDevice(&prev); }
+    ~CurrentDevice() { cudaSetDevice(prev); }
+};
+
+// waits for the work that may still read a registered base vector, then frees every replica on its own device
+static void free_bases(BaseSet* bs) {
+    CurrentDevice keep;
+    for (int s = 0; s < MAX_DEV; ++s) if (bs->t[s]) { cudaSetDevice(bs->t[s]->device); cudaDeviceSynchronize(); msm_table_free(bs->t[s]); delete bs->t[s]; }
+    delete bs;
+}
+
 struct TlCtx {
     Ctx* c[MAX_DEV] = {};
     uint64_t epoch = 0;
@@ -99,12 +113,11 @@ struct TlCtx {
         if (epoch != g_epoch.load() || !g_inited.load()) return;
         std::lock_guard<std::mutex> lk(g_mu);
         if (epoch != g_epoch.load()) return;
-        int cur = 0; cudaGetDevice(&cur);
+        CurrentDevice keep;
         for (int s = 0; s < MAX_DEV; ++s) if (c[s]) {
             for (size_t i = 0; i < g_ctxs.size(); ++i) if (g_ctxs[i] == c[s]) { g_ctxs.erase(g_ctxs.begin() + i); break; }
             c[s]->release(); delete c[s]; g_nctx--;
         }
-        cudaSetDevice(cur);
     }
 };
 static thread_local TlCtx tl;
@@ -176,6 +189,28 @@ static size_t call_budget() {
 }
 // host Fr values arrive with 8-byte alignment (Rust / C callers); Fr is alignas(16), so always copy bytewise
 static inline Fr as_fr(const b200_fr* p) { Fr r; memcpy(&r, p, sizeof r); return r; }
+
+// NTT pre / post scaling as the ABI passes it (mode 0 none, 1 constant c[0], 3 cycle c[i mod 3]); -1 on a bad mode or missing constants
+static int decode_scales(int pre_mode, const b200_fr* pre, int post_mode, const b200_fr* post, NttScale* a, NttScale* b) {
+    B200_CHECK((pre_mode == 0 || pre_mode == 1 || pre_mode == 3) && (post_mode == 0 || post_mode == 1 || post_mode == 3), -1, "ntt: scale mode must be 0, 1 or 3");
+    B200_CHECK((pre_mode == 0 || pre) && (post_mode == 0 || post), -1, "ntt: scale constants missing");
+    a->mode = pre_mode; b->mode = post_mode;
+    for (int i = 0; i < pre_mode; ++i) a->c[i] = as_fr(pre + i);
+    for (int i = 0; i < post_mode; ++i) b->c[i] = as_fr(post + i);
+    return 0;
+}
+// coeff_to_extended's pre-scale: coefficient i times zeta^(i mod 3) (zeta is a cube root of unity)
+static NttScale coset_scale(const Fr& zeta) {
+    NttScale s;
+    s.mode = 3; s.c[0] = fp_one<FrTag>(); s.c[1] = zeta; s.c[2] = zeta * zeta;
+    return s;
+}
+// extended_to_coeff's post-scale: the inverse transform's divisor times zeta^-(i mod 3), where zeta^-1 = zeta^2
+static NttScale coset_unscale(const Fr& zeta, const Fr& divisor) {
+    NttScale s;
+    s.mode = 3; s.c[0] = divisor; s.c[1] = divisor * (zeta * zeta); s.c[2] = divisor * zeta;
+    return s;
+}
 
 // ---- large host <-> device copies of PAGEABLE caller memory (what a Rust Vec<Fr> is) ------------------------------------------------
 // cudaMemcpyAsync from pageable memory runs at 6-7 GB/s on this box (one driver thread copying into its own staging buffer).  Here the
@@ -423,9 +458,7 @@ static int msm_host_on(Ctx* c, const BaseSet* bs, const b200_fr* const* cols, si
         if (int rc = msm_dev_on(c, bs, c->stage_a.as<Fr>(), n, n, nb, base_off, c->small.as<G1Xyzz>() + b0, ss.st)) return rc;
         if (b0 + nb < count) B200_CUDA(cudaStreamSynchronize(ss.st));      // the staging buffer is reused by the next sub-batch
     }
-    B200_CUDA(cudaMemcpyAsync(h_out, c->small.p, sizeof(G1Xyzz) * count, cudaMemcpyDeviceToHost, ss.st));
-    B200_CUDA(cudaStreamSynchronize(ss.st));
-    return 0;
+    return d2h_one(c, h_out, c->small.p, sizeof(G1Xyzz) * count, ss.st);
 }
 static void slice_bounds(size_t n, int g, int world, size_t* lo, size_t* hi) {
     const size_t base = n / world, rem = n % world;
@@ -504,17 +537,13 @@ void b200_shutdown(void) {
         delete g_workers[s]; g_workers[s] = nullptr;
     }
     std::lock_guard<std::mutex> lk(g_mu);
-    int cur = 0; cudaGetDevice(&cur);
-    for (auto& kv : g_tables) {
-        for (int s = 0; s < MAX_DEV; ++s) if (kv.second->t[s]) { cudaSetDevice(kv.second->t[s]->device); msm_table_free(kv.second->t[s]); delete kv.second->t[s]; }
-        delete kv.second;
-    }
+    CurrentDevice keep;
+    for (auto& kv : g_tables) free_bases(kv.second);
     g_tables.clear();
     for (Ctx* c : g_ctxs) { c->release(); delete c; }          // streams and scratch of every calling thread, alive or not
     g_ctxs.clear(); g_nctx.store(0);
     g_epoch++;
     for (int s = 0; s < g_ndev.load(); ++s) { cudaSetDevice(g_devs[s].id); g_devs[s].ntt.release(); g_devs[s].id = -1; }
-    cudaSetDevice(cur);
     g_ndev.store(0);
 }
 
@@ -528,9 +557,10 @@ int b200_profile_enable(int on) {
 }
 int b200_profile_read(int cls, double* total_ms, uint64_t* count) {
     B200_CHECK(cls >= 0 && cls < PROF_NCLASS && total_ms && count, -1, "profile_read: bad argument");
-    int cur = 0; cudaGetDevice(&cur);
-    for (int s = 0; s < g_ndev.load(); ++s) { B200_CUDA(cudaSetDevice(g_devs[s].id)); B200_CUDA(cudaDeviceSynchronize()); }
-    cudaSetDevice(cur);
+    {
+        CurrentDevice keep;
+        for (int s = 0; s < g_ndev.load(); ++s) { B200_CUDA(cudaSetDevice(g_devs[s].id)); B200_CUDA(cudaDeviceSynchronize()); }
+    }
     std::lock_guard<std::mutex> lk(g_prof_mu);
     double ms = 0; uint64_t n = 0;
     for (auto& r : g_prof_recs) if (r.cls == cls) { float t = 0; if (cudaEventElapsedTime(&t, r.e0, r.e1) == cudaSuccess) { ms += t; ++n; } else cudaGetLastError(); }
@@ -577,20 +607,15 @@ int b200_sync_all(void) {
 }
 
 // ---- bases ---------------------------------------------------------------------------------------------------
-int b200_bases_register_dev(const void* d_bases, size_t n, int window_bits, uint64_t* handle) {
-    B200_ENTER(c, d_bases);
+// device base vector on the context's device -> handle of its window table, built there and replicated to the other devices
+static int bases_register_on(Ctx* c, const G1Affine* d_bases, size_t n, int window_bits, uint64_t* handle, cudaStream_t st) {
     B200_CHECK(d_bases && handle && n > 0, -1, "bases_register: null argument or n == 0");
     B200_CHECK(window_bits == 0 || (window_bits >= 4 && window_bits <= 24), -1, "bases_register: window_bits %d not in {0, 4..24}", window_bits);
     BaseSet* bs = new BaseSet();
-    auto fail = [&](int rc) {
-        int cur = 0; cudaGetDevice(&cur);
-        for (int s = 0; s < MAX_DEV; ++s) if (bs->t[s]) { cudaSetDevice(bs->t[s]->device); msm_table_free(bs->t[s]); delete bs->t[s]; }
-        cudaSetDevice(cur);
-        delete bs; return rc;
-    };
+    auto fail = [&](int rc) { free_bases(bs); return rc; };
     MsmTable* t = new MsmTable();
     bs->t[c->slot] = t;
-    if (int rc = msm_table_build(t, reinterpret_cast<const G1Affine*>(d_bases), n, window_bits, c->stream)) return fail(rc);
+    if (int rc = msm_table_build(t, d_bases, n, window_bits, st)) return fail(rc);
     g_launches += (uint64_t)(t->W - 1);
     bs->n = n; bs->c = t->c; bs->W = t->W;
     // replicas: the finished table crosses NVLink once per extra device (cheaper than rebuilding: one inversion per point and level)
@@ -598,26 +623,35 @@ int b200_bases_register_dev(const void* d_bases, size_t n, int window_bits, uint
         MsmTable* r = new MsmTable();
         *r = *t; r->d_table = nullptr; r->device = g_devs[s].id;
         bs->t[s] = r;
-        cudaSetDevice(r->device);
-        cudaError_t e = cudaMalloc(&r->d_table, sizeof(G1Affine) * n * t->W);
-        cudaSetDevice(c->dev);
+        cudaError_t e;
+        {
+            CurrentDevice keep;
+            cudaSetDevice(r->device);
+            e = cudaMalloc(&r->d_table, sizeof(G1Affine) * n * t->W);
+        }
         if (e != cudaSuccess) { set_error("bases_register: replica on device %d: %s", r->device, cudaGetErrorString(e)); return fail(-2); }
-        e = cudaMemcpyPeerAsync(r->d_table, r->device, t->d_table, t->device, sizeof(G1Affine) * n * t->W, c->stream);
+        e = cudaMemcpyPeerAsync(r->d_table, r->device, t->d_table, t->device, sizeof(G1Affine) * n * t->W, st);
         if (e != cudaSuccess) { set_error("bases_register: peer copy: %s", cudaGetErrorString(e)); return fail(-2); }
     }
-    cudaError_t e = cudaStreamSynchronize(c->stream);
+    cudaError_t e = cudaStreamSynchronize(st);
     if (e != cudaSuccess) { set_error("bases_register: %s", cudaGetErrorString(e)); return fail(-2); }
     std::lock_guard<std::mutex> lk(g_mu);
     *handle = g_next_handle++;
     g_tables[*handle] = bs;
     return 0;
 }
+int b200_bases_register_dev(const void* d_bases, size_t n, int window_bits, uint64_t* handle) {
+    B200_ENTER(c, d_bases);
+    StreamScope ss(c, nullptr);
+    return bases_register_on(c, reinterpret_cast<const G1Affine*>(d_bases), n, window_bits, handle, ss.st);
+}
 int b200_bases_register(const b200_g1_affine* bases, size_t n, int window_bits, uint64_t* handle) {
     B200_ENTER(c, nullptr);
     B200_CHECK(bases && handle && n > 0, -1, "bases_register: null argument or n == 0");
     if (c->stage_a.ensure(sizeof(G1Affine) * n)) return -2;
-    B200_CUDA(cudaMemcpyAsync(c->stage_a.p, bases, sizeof(G1Affine) * n, cudaMemcpyHostToDevice, c->stream));
-    return b200_bases_register_dev(c->stage_a.p, n, window_bits, handle);
+    StreamScope ss(c, nullptr);
+    if (int rc = h2d_one(c, c->stage_a.p, bases, sizeof(G1Affine) * n, ss.st)) return rc;
+    return bases_register_on(c, c->stage_a.as<G1Affine>(), n, window_bits, handle, ss.st);
 }
 int b200_bases_release(uint64_t handle) {
     CallGuard cg; if (!cg.ok) return -3;
@@ -629,10 +663,7 @@ int b200_bases_release(uint64_t handle) {
         bs = it->second;
         g_tables.erase(it);
     }
-    int cur = 0; cudaGetDevice(&cur);
-    for (int s = 0; s < MAX_DEV; ++s) if (bs->t[s]) { cudaSetDevice(bs->t[s]->device); cudaDeviceSynchronize(); msm_table_free(bs->t[s]); delete bs->t[s]; }
-    cudaSetDevice(cur);
-    delete bs;
+    free_bases(bs);
     return 0;
 }
 int b200_bases_info(uint64_t handle, size_t* n, int* window_bits, int* windows) {
@@ -701,6 +732,13 @@ int b200_msm(uint64_t bases, const b200_fr* scalars, size_t n, b200_g1_jac* out)
     const b200_fr* cols[1] = {scalars};
     return b200_msm_batch(bases, cols, n, 1, out);
 }
+// out[g] = sum of points[g * count .. (g + 1) * count)
+static int g1_sum_on(const G1Xyzz* pts, size_t groups, size_t count, G1Xyzz* out, cudaStream_t st) {
+    B200_CHECK(pts && out, -1, "g1_sum: null pointer");
+    int rc = g1_sum_run(pts, groups, count, out, st);
+    if (!rc) g_launches += 1;
+    return rc;
+}
 // base-split MSM on device-resident slices (north star: bases split across the GPUs, partial sums reduced over NVLink)
 int b200_msm_sharded_dev(uint64_t bases, const void* const* d_scalar_slices, size_t n, size_t batch, b200_g1_jac* out) {
     CallGuard cg; if (!cg.ok) return -3;
@@ -711,7 +749,7 @@ int b200_msm_sharded_dev(uint64_t bases, const void* const* d_scalar_slices, siz
     B200_CHECK(n <= t->n && batch >= 1 && batch <= 4096, -1, "msm_sharded: bad sizes");
     Ctx* cs[MAX_DEV];
     for (int s = 0; s < nd; ++s) if (int rc = get_ctx(&cs[s], s)) return rc;
-    int cur = 0; cudaGetDevice(&cur);
+    CurrentDevice keep;
     // gather buffer on device 0: [column][device] XYZZ partials
     if (cs[0]->small.ensure(sizeof(G1Xyzz) * batch * (nd + 2))) return -2;
     G1Xyzz* gather = cs[0]->small.as<G1Xyzz>();
@@ -721,8 +759,8 @@ int b200_msm_sharded_dev(uint64_t bases, const void* const* d_scalar_slices, siz
         B200_CUDA(cudaSetDevice(cs[s]->dev));
         StreamScope ss(cs[s], nullptr);
         G1Xyzz* part = gather + batch * nd;           // device 0: a staging row behind the gather matrix
-        if (s != 0) { if (cs[s]->small.ensure(sizeof(G1Xyzz) * batch)) { cudaSetDevice(cur); return -2; } part = cs[s]->small.as<G1Xyzz>(); }
-        if (int rc = msm_dev_on(cs[s], t, reinterpret_cast<const Fr*>(d_scalar_slices[s]), hi - lo, hi - lo, batch, lo, part, ss.st)) { cudaSetDevice(cur); return rc; }
+        if (s != 0) { if (cs[s]->small.ensure(sizeof(G1Xyzz) * batch)) return -2; part = cs[s]->small.as<G1Xyzz>(); }
+        if (int rc = msm_dev_on(cs[s], t, reinterpret_cast<const Fr*>(d_scalar_slices[s]), hi - lo, hi - lo, batch, lo, part, ss.st)) return rc;
         // partial sums travel to device 0 over NVLink: column b of device s lands at gather[b * nd + s]
         B200_CUDA(cudaMemcpy2DAsync(gather + s, sizeof(G1Xyzz) * nd, part, sizeof(G1Xyzz), sizeof(G1Xyzz), batch, cudaMemcpyDefault, ss.st));
     }
@@ -732,44 +770,41 @@ int b200_msm_sharded_dev(uint64_t bases, const void* const* d_scalar_slices, siz
     {
         StreamScope ss(cs[0], nullptr);
         G1Xyzz* sums = gather + batch * (nd + 1);
-        if (int rc = g1_sum_run(gather, batch, nd, sums, ss.st)) { cudaSetDevice(cur); return rc; }
-        g_launches += 1;
+        if (int rc = g1_sum_on(gather, batch, nd, sums, ss.st)) return rc;
         B200_CUDA(cudaMemcpyAsync(h.data(), sums, sizeof(G1Xyzz) * batch, cudaMemcpyDeviceToHost, ss.st));
         B200_CUDA(cudaStreamSynchronize(ss.st));
     }
-    cudaSetDevice(cur);
     normalize_host(h.data(), batch, out);
     return 0;
 }
 int b200_g1_sum_dev(const void* d_points_xyzz, size_t groups, size_t count, void* d_out_xyzz, void* stream) {
     B200_ENTER(c, d_points_xyzz);
-    B200_CHECK(d_points_xyzz && d_out_xyzz, -1, "g1_sum: null pointer");
     StreamScope ss(c, stream);
-    int rc = g1_sum_run(reinterpret_cast<const G1Xyzz*>(d_points_xyzz), groups, count, reinterpret_cast<G1Xyzz*>(d_out_xyzz), ss.st);
-    if (!rc) g_launches += 1;
+    return g1_sum_on(reinterpret_cast<const G1Xyzz*>(d_points_xyzz), groups, count, reinterpret_cast<G1Xyzz*>(d_out_xyzz), ss.st);
+}
+static int g1_fft_on(Ctx* c, const G1Affine* in, uint32_t log_n, const b200_fr* omega, const b200_fr* scale, G1Affine* out, cudaStream_t st) {
+    B200_CHECK(in && omega && out, -1, "g1_fft: null pointer");
+    const Fr w = as_fr(omega);
+    Fr sc = fp_one<FrTag>();
+    if (scale) sc = as_fr(scale);
+    int rc = g1_fft_run(in, log_n, w, scale ? &sc : nullptr, out, c->msm_ws.misc, st);
+    if (!rc) g_launches += (uint64_t)g1_fft_launches(log_n);
     return rc;
 }
 int b200_g1_fft_dev(const void* d_in_affine, uint32_t log_n, const b200_fr* omega, const b200_fr* scale, void* d_out_affine, void* stream) {
     B200_ENTER(c, d_in_affine);
-    B200_CHECK(d_in_affine && omega && d_out_affine, -1, "g1_fft: null pointer");
-    const Fr w = as_fr(omega);
-    Fr sc = fp_one<FrTag>();
-    if (scale) sc = as_fr(scale);
     StreamScope ss(c, stream);
-    int rc = g1_fft_run(reinterpret_cast<const G1Affine*>(d_in_affine), log_n, w, scale ? &sc : nullptr, reinterpret_cast<G1Affine*>(d_out_affine), c->msm_ws.misc, ss.st);
-    if (!rc) g_launches += (uint64_t)g1_fft_launches(log_n);
-    return rc;
+    return g1_fft_on(c, reinterpret_cast<const G1Affine*>(d_in_affine), log_n, omega, scale, reinterpret_cast<G1Affine*>(d_out_affine), ss.st);
 }
 int b200_g1_fft(const b200_g1_affine* in, uint32_t log_n, const b200_fr* omega, const b200_fr* scale, b200_g1_affine* out) {
     B200_ENTER(c, nullptr);
     B200_CHECK(in && omega && out && log_n <= 26, -1, "g1_fft: bad argument");
-    const size_t n = (size_t)1 << log_n;
-    if (c->stage_a.ensure(sizeof(G1Affine) * n) || c->stage_b.ensure(sizeof(G1Affine) * n)) return -2;
-    B200_CUDA(cudaMemcpyAsync(c->stage_a.p, in, sizeof(G1Affine) * n, cudaMemcpyHostToDevice, c->stream));
-    if (int rc = b200_g1_fft_dev(c->stage_a.p, log_n, omega, scale, c->stage_b.p, nullptr)) return rc;
-    B200_CUDA(cudaMemcpyAsync(out, c->stage_b.p, sizeof(G1Affine) * n, cudaMemcpyDeviceToHost, c->stream));
-    B200_CUDA(cudaStreamSynchronize(c->stream));
-    return 0;
+    const size_t bytes = sizeof(G1Affine) << log_n;
+    if (c->stage_a.ensure(bytes) || c->stage_b.ensure(bytes)) return -2;
+    StreamScope ss(c, nullptr);
+    if (int rc = h2d_one(c, c->stage_a.p, in, bytes, ss.st)) return rc;
+    if (int rc = g1_fft_on(c, c->stage_a.as<G1Affine>(), log_n, omega, scale, c->stage_b.as<G1Affine>(), ss.st)) return rc;
+    return d2h_one(c, out, c->stage_b.p, bytes, ss.st);
 }
 int b200_g1_fixed_base_mul_dev(const void* d_scalars, size_t n, const b200_g1_affine* base, void* d_out_affine, void* stream) {
     B200_ENTER(c, d_scalars);
@@ -802,13 +837,9 @@ int b200_ntt_dev(const void* d_src, size_t src_stride, size_t n_in, void* d_tmp,
                  const b200_fr* omega, int pre_mode, const b200_fr* pre, int post_mode, const b200_fr* post, size_t batch, void* stream) {
     B200_ENTER(c, d_src);
     B200_CHECK(d_src && d_tmp && d_dst && omega, -1, "ntt: null pointer");
-    B200_CHECK((pre_mode == 0 || pre_mode == 1 || pre_mode == 3) && (post_mode == 0 || post_mode == 1 || post_mode == 3), -1, "ntt: scale mode must be 0, 1 or 3");
-    B200_CHECK((pre_mode == 0 || pre) && (post_mode == 0 || post), -1, "ntt: scale constants missing");
-    if (batch == 0) return 0;
     NttScale a, b;
-    a.mode = pre_mode; b.mode = post_mode;
-    for (int i = 0; i < pre_mode; ++i) a.c[i] = as_fr(pre + i);
-    for (int i = 0; i < post_mode; ++i) b.c[i] = as_fr(post + i);
+    if (int rc = decode_scales(pre_mode, pre, post_mode, post, &a, &b)) return rc;
+    if (batch == 0) return 0;
     StreamScope ss(c, stream);
     return ntt_call(c, reinterpret_cast<const Fr*>(d_src), src_stride, n_in, reinterpret_cast<Fr*>(d_tmp), reinterpret_cast<Fr*>(d_dst), dst_stride,
                     log_n, as_fr(omega), a, b, (int)batch, ss.st);
@@ -821,15 +852,16 @@ int b200_ntt_dev(const void* d_src, size_t src_stride, size_t n_in, void* d_tmp,
 static int ntt_sharded_on(Ctx* const* cs, int nd, const Fr* const* src, Fr* const* tmp, Fr* const* dst, uint32_t log_n, uint64_t n_in, const Fr& omega,
                           const NttScale& pre, const NttScale& post) {
     NttPlan* plans[MAX_DEV]; int ids[MAX_DEV]; cudaStream_t st[MAX_DEV]; cudaEvent_t ev[MAX_DEV];
-    int cur = 0; cudaGetDevice(&cur);
-    for (int s = 0; s < nd; ++s) {
-        cudaSetDevice(cs[s]->dev);
-        plans[s] = warm_plan(s, log_n, omega, cs[s]->stream);
-        if (!plans[s]) { cudaSetDevice(cur); return -2; }
-        ids[s] = cs[s]->dev; st[s] = cs[s]->stream; ev[s] = cs[s]->last_ev;
-        if (cs[s]->has_last && cs[s]->last_stream != st[s]) cudaStreamWaitEvent(st[s], cs[s]->last_ev, 0);
+    {
+        CurrentDevice keep;
+        for (int s = 0; s < nd; ++s) {
+            cudaSetDevice(cs[s]->dev);
+            plans[s] = warm_plan(s, log_n, omega, cs[s]->stream);
+            if (!plans[s]) return -2;
+            ids[s] = cs[s]->dev; st[s] = cs[s]->stream; ev[s] = cs[s]->last_ev;
+            if (cs[s]->has_last && cs[s]->last_stream != st[s]) cudaStreamWaitEvent(st[s], cs[s]->last_ev, 0);
+        }
     }
-    cudaSetDevice(cur);
     int rc = ntt_run_sharded(plans, nd, ids, src, tmp, dst, log_n, omega, pre, post, n_in, st, ev);
     for (int s = 0; s < nd && !rc; ++s) { cs[s]->last_stream = st[s]; cs[s]->has_last = true; }       // ev[s] was recorded after the last pass
     if (!rc) g_launches += (uint64_t)ntt_launches_per_run(log_n) * nd;
@@ -841,12 +873,8 @@ int b200_ntt_sharded_dev(const void* const* d_src_slices, void* const* d_tmp_sli
     const int nd = g_ndev.load();
     B200_CHECK(nd >= 2, -1, "ntt_sharded: needs a multi-device process (b200_init_multi)");
     B200_CHECK(d_src_slices && d_tmp_slices && d_dst_slices && omega, -1, "ntt_sharded: null pointer");
-    B200_CHECK((pre_mode == 0 || pre_mode == 1 || pre_mode == 3) && (post_mode == 0 || post_mode == 1 || post_mode == 3), -1, "ntt: scale mode must be 0, 1 or 3");
-    B200_CHECK((pre_mode == 0 || pre) && (post_mode == 0 || post), -1, "ntt: scale constants missing");
     NttScale a, b;
-    a.mode = pre_mode; b.mode = post_mode;
-    for (int i = 0; i < pre_mode; ++i) a.c[i] = as_fr(pre + i);
-    for (int i = 0; i < post_mode; ++i) b.c[i] = as_fr(post + i);
+    if (int rc = decode_scales(pre_mode, pre, post_mode, post, &a, &b)) return rc;
     Ctx* cs[MAX_DEV];
     for (int s = 0; s < nd; ++s) {
         if (int rc = get_ctx(&cs[s], s)) return rc;
@@ -881,12 +909,13 @@ static int ntt_host_on(Ctx* c, const b200_fr* const* src, b200_fr* const* dst, s
     }
     return 0;
 }
-// shared host path: on a multi-device process a batch is dealt over the devices; a single large transform is sharded
-static int ntt_host(const b200_fr* const* src, b200_fr* const* dst, size_t batch, size_t n_in, uint32_t log_n, const Fr& omega,
+// shared host path: on a multi-device process a batch is dealt over the devices; a single large transform is sharded.
+// n_in_or_null: input elements per polynomial, NULL = 2^log_n
+static int ntt_host(const b200_fr* const* src, b200_fr* const* dst, size_t batch, const size_t* n_in_or_null, uint32_t log_n, const Fr& omega,
                     const NttScale& pre, const NttScale& post) {
     B200_ENTER(c, nullptr);
     B200_CHECK(log_n >= 1 && log_n <= 28, -1, "ntt: log_n = %u out of range [1, 28]", log_n);
-    const size_t N = (size_t)1 << log_n;
+    const size_t N = (size_t)1 << log_n, n_in = n_in_or_null ? *n_in_or_null : N;
     B200_CHECK(n_in <= N, -1, "ntt: %zu input elements > 2^%u", n_in, log_n);
     if (batch == 0) return 0;
     const int nd = g_ndev.load();
@@ -932,14 +961,14 @@ static int ntt_host(const b200_fr* const* src, b200_fr* const* dst, size_t batch
 int b200_fft_batch(b200_fr* const* a, size_t batch, uint32_t log_n, const b200_fr* omega) {
     B200_CHECK(a && omega, -1, "fft: null pointer");
     NttScale none;
-    return ntt_host(a, a, batch, (size_t)1 << (log_n <= 28 ? log_n : 0), log_n, as_fr(omega), none, none);
+    return ntt_host(a, a, batch, nullptr, log_n, as_fr(omega), none, none);
 }
 int b200_fft(b200_fr* a, uint32_t log_n, const b200_fr* omega) { b200_fr* p[1] = {a}; return b200_fft_batch(p, 1, log_n, omega); }
 int b200_ifft_batch(b200_fr* const* a, size_t batch, uint32_t log_n, const b200_fr* omega_inv, const b200_fr* divisor) {
     B200_CHECK(a && omega_inv && divisor, -1, "ifft: null pointer");
     NttScale none, post;
     post.mode = 1; post.c[0] = as_fr(divisor);
-    return ntt_host(a, a, batch, (size_t)1 << (log_n <= 28 ? log_n : 0), log_n, as_fr(omega_inv), none, post);
+    return ntt_host(a, a, batch, nullptr, log_n, as_fr(omega_inv), none, post);
 }
 int b200_ifft(b200_fr* a, uint32_t log_n, const b200_fr* omega_inv, const b200_fr* divisor) {
     b200_fr* p[1] = {a};
@@ -947,9 +976,8 @@ int b200_ifft(b200_fr* a, uint32_t log_n, const b200_fr* omega_inv, const b200_f
 }
 int b200_coeff_to_extended_batch(const b200_fr* const* coeffs, size_t batch, size_t n_coeffs, uint32_t ext_k, const b200_fr* ext_omega, const b200_fr* zeta, b200_fr* const* out) {
     B200_CHECK(coeffs && out && ext_omega && zeta, -1, "coeff_to_extended: null pointer");
-    NttScale pre, none;
-    pre.mode = 3; pre.c[0] = fp_one<FrTag>(); pre.c[1] = as_fr(zeta); pre.c[2] = as_fr(zeta) * as_fr(zeta);
-    return ntt_host(coeffs, out, batch, n_coeffs, ext_k, as_fr(ext_omega), pre, none);
+    NttScale none;
+    return ntt_host(coeffs, out, batch, &n_coeffs, ext_k, as_fr(ext_omega), coset_scale(as_fr(zeta)), none);
 }
 int b200_coeff_to_extended(const b200_fr* coeffs, size_t n_coeffs, uint32_t ext_k, const b200_fr* ext_omega, const b200_fr* zeta, b200_fr* out) {
     const b200_fr* s[1] = {coeffs}; b200_fr* d[1] = {out};
@@ -957,24 +985,25 @@ int b200_coeff_to_extended(const b200_fr* coeffs, size_t n_coeffs, uint32_t ext_
 }
 int b200_extended_to_coeff(b200_fr* a, uint32_t ext_k, const b200_fr* ext_omega_inv, const b200_fr* ext_ifft_divisor, const b200_fr* zeta) {
     B200_CHECK(a && ext_omega_inv && ext_ifft_divisor && zeta, -1, "extended_to_coeff: null pointer");
-    NttScale none, post;
-    const Fr z = as_fr(zeta), z2 = z * z, d = as_fr(ext_ifft_divisor);
-    post.mode = 3; post.c[0] = d; post.c[1] = d * z2; post.c[2] = d * z;     // zeta^-1 = zeta^2
+    NttScale none;
     b200_fr* p[1] = {a};
-    return ntt_host(p, p, 1, (size_t)1 << (ext_k <= 28 ? ext_k : 0), ext_k, as_fr(ext_omega_inv), none, post);
+    return ntt_host(p, p, 1, nullptr, ext_k, as_fr(ext_omega_inv), none, coset_unscale(as_fr(zeta), as_fr(ext_ifft_divisor)));
 }
 
 // ---- polynomial ops --------------------------------------------------------------------------------------------
-int b200_poly_op_dev(int op, const void* d_a, const void* d_b, const b200_fr* s, void* d_out, size_t n, void* stream) {
-    B200_ENTER(c, d_a);
+static int poly_op_on(int op, const Fr* a, const Fr* b, const b200_fr* s, Fr* out, size_t n, cudaStream_t st) {
     B200_CHECK(op >= 0 && op <= 4, -1, "poly_op: unknown op %d", op);
-    B200_CHECK(d_a && d_out && (op == POLY_SCALE || d_b) && (op < POLY_SCALE || s), -1, "poly_op: missing operand for op %d", op);
+    B200_CHECK(a && out && (op == POLY_SCALE || b) && (op < POLY_SCALE || s), -1, "poly_op: missing operand for op %d", op);
     Fr sv = fp_zero<FrTag>();
     if (s) sv = as_fr(s);
-    StreamScope ss(c, stream);
-    int rc = poly_binary(op, reinterpret_cast<const Fr*>(d_a), reinterpret_cast<const Fr*>(d_b), s ? &sv : nullptr, reinterpret_cast<Fr*>(d_out), n, ss.st);
+    int rc = poly_binary(op, a, b, s ? &sv : nullptr, out, n, st);
     if (!rc && n) g_launches += 1;
     return rc;
+}
+int b200_poly_op_dev(int op, const void* d_a, const void* d_b, const b200_fr* s, void* d_out, size_t n, void* stream) {
+    B200_ENTER(c, d_a);
+    StreamScope ss(c, stream);
+    return poly_op_on(op, reinterpret_cast<const Fr*>(d_a), reinterpret_cast<const Fr*>(d_b), s, reinterpret_cast<Fr*>(d_out), n, ss.st);
 }
 int b200_poly_op(int op, const b200_fr* a, const b200_fr* b, const b200_fr* s, b200_fr* out, size_t n) {
     B200_ENTER(c, nullptr);
@@ -983,77 +1012,83 @@ int b200_poly_op(int op, const b200_fr* a, const b200_fr* b, const b200_fr* s, b
     const bool need_b = op != POLY_SCALE;
     B200_CHECK(!need_b || b, -1, "poly_op: missing operand b");
     if (c->stage_a.ensure(sizeof(Fr) * n) || (need_b && c->stage_b.ensure(sizeof(Fr) * n))) return -2;
-    B200_CUDA(cudaMemcpyAsync(c->stage_a.p, a, sizeof(Fr) * n, cudaMemcpyHostToDevice, c->stream));
-    if (need_b) B200_CUDA(cudaMemcpyAsync(c->stage_b.p, b, sizeof(Fr) * n, cudaMemcpyHostToDevice, c->stream));
-    if (int rc = b200_poly_op_dev(op, c->stage_a.p, need_b ? c->stage_b.p : nullptr, s, c->stage_a.p, n, nullptr)) return rc;
-    B200_CUDA(cudaMemcpyAsync(out, c->stage_a.p, sizeof(Fr) * n, cudaMemcpyDeviceToHost, c->stream));
-    B200_CUDA(cudaStreamSynchronize(c->stream));
-    return 0;
+    StreamScope ss(c, nullptr);
+    if (int rc = h2d_one(c, c->stage_a.p, a, sizeof(Fr) * n, ss.st)) return rc;
+    if (need_b) { if (int rc = h2d_one(c, c->stage_b.p, b, sizeof(Fr) * n, ss.st)) return rc; }
+    if (int rc = poly_op_on(op, c->stage_a.as<Fr>(), need_b ? c->stage_b.as<Fr>() : nullptr, s, c->stage_a.as<Fr>(), n, ss.st)) return rc;
+    return d2h_one(c, out, c->stage_a.p, sizeof(Fr) * n, ss.st);
+}
+// d_polys: host array of device addresses
+static int lincomb_on(Ctx* c, const Fr* const* d_polys, const b200_fr* scalars, size_t count, size_t n, Fr* out, cudaStream_t st) {
+    B200_CHECK(out && (count == 0 || (d_polys && scalars)), -1, "poly_lincomb: null pointer");
+    std::vector<Fr> sv(count);
+    if (count) memcpy(sv.data(), scalars, sizeof(Fr) * count);
+    int rc = poly_lincomb(d_polys, sv.data(), count, out, n, c->poly_ws, st);
+    if (!rc && n) g_launches += 1;
+    return rc;
 }
 int b200_poly_lincomb_dev(const void* const* d_polys, const b200_fr* scalars, size_t count, size_t n, void* d_out, void* stream) {
     B200_ENTER(c, d_out);
-    B200_CHECK(d_out && (count == 0 || (d_polys && scalars)), -1, "poly_lincomb: null pointer");
-    std::vector<Fr> sv(count);
-    if (count) memcpy(sv.data(), scalars, sizeof(Fr) * count);
     StreamScope ss(c, stream);
-    int rc = poly_lincomb(reinterpret_cast<const Fr* const*>(d_polys), sv.data(), count, reinterpret_cast<Fr*>(d_out), n, c->poly_ws, ss.st);
-    if (!rc && n) g_launches += 1;
-    return rc;
+    return lincomb_on(c, reinterpret_cast<const Fr* const*>(d_polys), scalars, count, n, reinterpret_cast<Fr*>(d_out), ss.st);
 }
 int b200_poly_lincomb(const b200_fr* const* polys, const b200_fr* scalars, size_t count, size_t n, b200_fr* out) {
     B200_ENTER(c, nullptr);
     B200_CHECK(out && (count == 0 || (polys && scalars)), -1, "poly_lincomb: null pointer");
     if (n == 0) return 0;
     if (c->stage_a.ensure(sizeof(Fr) * n * (count ? count : 1)) || c->stage_b.ensure(sizeof(Fr) * n)) return -2;
-    std::vector<const void*> ptrs(count);
+    std::vector<const Fr*> ptrs(count);
     std::vector<HostSeg> up(count);
     for (size_t j = 0; j < count; ++j) {
         B200_CHECK(polys[j], -1, "poly_lincomb: polys[%zu] is null", j);
         ptrs[j] = c->stage_a.as<Fr>() + j * n;
         up[j] = HostSeg{(uint8_t*)const_cast<b200_fr*>(polys[j]), sizeof(Fr) * n};
     }
-    if (int rc = h2d_segments(c, c->stage_a.p, up.data(), count, c->stream)) return rc;
-    if (int rc = b200_poly_lincomb_dev(ptrs.data(), scalars, count, n, c->stage_b.p, nullptr)) return rc;
-    B200_CUDA(cudaMemcpyAsync(out, c->stage_b.p, sizeof(Fr) * n, cudaMemcpyDeviceToHost, c->stream));
-    B200_CUDA(cudaStreamSynchronize(c->stream));
-    return 0;
+    StreamScope ss(c, nullptr);
+    if (int rc = h2d_segments(c, c->stage_a.p, up.data(), count, ss.st)) return rc;
+    if (int rc = lincomb_on(c, ptrs.data(), scalars, count, n, c->stage_b.as<Fr>(), ss.st)) return rc;
+    return d2h_one(c, out, c->stage_b.p, sizeof(Fr) * n, ss.st);
 }
-int b200_poly_scale_cycle_dev(void* d_a, size_t n, const b200_fr* consts, uint32_t period, void* stream) {
-    B200_ENTER(c, d_a);
-    B200_CHECK(d_a && consts && period > 0 && period <= 1024, -1, "poly_scale_cycle: bad argument");
-    StreamScope ss(c, stream);
-    cudaStream_t st = ss.st;
+static int scale_cycle_on(Ctx* c, Fr* a, size_t n, const b200_fr* consts, uint32_t period, cudaStream_t st) {
+    B200_CHECK(a && consts && period > 0 && period <= 1024, -1, "poly_scale_cycle: bad argument");
     const Fr* d_consts = reinterpret_cast<const Fr*>(c->ring.push(consts, sizeof(Fr) * period, st));
     if (!d_consts) {
         if (c->small.ensure(sizeof(Fr) * period)) return -2;
-        B200_CUDA(cudaMemcpyAsync(c->small.p, consts, sizeof(Fr) * period, cudaMemcpyHostToDevice, st));
+        if (int rc = h2d_one(c, c->small.p, consts, sizeof(Fr) * period, st)) return rc;
         d_consts = c->small.as<Fr>();
     }
-    int rc = poly_scale_cycle(reinterpret_cast<const Fr*>(d_a), d_consts, period, reinterpret_cast<Fr*>(d_a), n, st);
+    int rc = poly_scale_cycle(a, d_consts, period, a, n, st);
     if (!rc && n) g_launches += 1;
     return rc;
+}
+int b200_poly_scale_cycle_dev(void* d_a, size_t n, const b200_fr* consts, uint32_t period, void* stream) {
+    B200_ENTER(c, d_a);
+    StreamScope ss(c, stream);
+    return scale_cycle_on(c, reinterpret_cast<Fr*>(d_a), n, consts, period, ss.st);
 }
 int b200_poly_scale_cycle(b200_fr* a, size_t n, const b200_fr* consts, uint32_t period) {
     B200_ENTER(c, nullptr);
     B200_CHECK(a && consts, -1, "poly_scale_cycle: null pointer");
     if (n == 0) return 0;
     if (c->stage_a.ensure(sizeof(Fr) * n)) return -2;
-    B200_CUDA(cudaMemcpyAsync(c->stage_a.p, a, sizeof(Fr) * n, cudaMemcpyHostToDevice, c->stream));
-    if (int rc = b200_poly_scale_cycle_dev(c->stage_a.p, n, consts, period, nullptr)) return rc;
-    B200_CUDA(cudaMemcpyAsync(a, c->stage_a.p, sizeof(Fr) * n, cudaMemcpyDeviceToHost, c->stream));
-    B200_CUDA(cudaStreamSynchronize(c->stream));
-    return 0;
+    StreamScope ss(c, nullptr);
+    if (int rc = h2d_one(c, c->stage_a.p, a, sizeof(Fr) * n, ss.st)) return rc;
+    if (int rc = scale_cycle_on(c, c->stage_a.as<Fr>(), n, consts, period, ss.st)) return rc;
+    return d2h_one(c, a, c->stage_a.p, sizeof(Fr) * n, ss.st);
 }
-int b200_poly_eval_batch_dev(const void* d_polys, size_t stride, size_t n, const b200_fr* x, size_t batch, void* d_out, void* stream) {
-    B200_ENTER(c, d_polys);
-    B200_CHECK(d_polys && x && d_out, -1, "poly_eval: null pointer");
+static int poly_eval_on(Ctx* c, const Fr* polys, size_t stride, size_t n, const b200_fr* x, size_t batch, Fr* out, cudaStream_t st) {
+    B200_CHECK(polys && x && out, -1, "poly_eval: null pointer");
     if (batch == 0) return 0;
     std::vector<Fr> xv(batch);
     memcpy(xv.data(), x, sizeof(Fr) * batch);
-    StreamScope ss(c, stream);
-    int rc = poly_eval(reinterpret_cast<const Fr*>(d_polys), stride, n, xv.data(), reinterpret_cast<Fr*>(d_out), (int)batch, c->poly_ws, ss.st);
+    int rc = poly_eval(polys, stride, n, xv.data(), out, (int)batch, c->poly_ws, st);
     if (!rc && n) g_launches += 2;
     return rc;
+}
+int b200_poly_eval_batch_dev(const void* d_polys, size_t stride, size_t n, const b200_fr* x, size_t batch, void* d_out, void* stream) {
+    B200_ENTER(c, d_polys);
+    StreamScope ss(c, stream);
+    return poly_eval_on(c, reinterpret_cast<const Fr*>(d_polys), stride, n, x, batch, reinterpret_cast<Fr*>(d_out), ss.st);
 }
 int b200_poly_eval_batch(const b200_fr* const* polys, size_t n, const b200_fr* x, size_t batch, b200_fr* out) {
     B200_ENTER(c, nullptr);
@@ -1065,75 +1100,79 @@ int b200_poly_eval_batch(const b200_fr* const* polys, size_t n, const b200_fr* x
         B200_CHECK(n == 0 || polys[p], -1, "poly_eval: polys[%zu] is null", p);
         up[p] = HostSeg{(uint8_t*)const_cast<b200_fr*>(polys[p]), sizeof(Fr) * n};
     }
-    if (n) { if (int rc = h2d_segments(c, c->stage_a.p, up.data(), batch, c->stream)) return rc; }
-    if (int rc = b200_poly_eval_batch_dev(c->stage_a.p, n, n, x, batch, c->small.p, nullptr)) return rc;
-    B200_CUDA(cudaMemcpyAsync(out, c->small.p, sizeof(Fr) * batch, cudaMemcpyDeviceToHost, c->stream));
-    B200_CUDA(cudaStreamSynchronize(c->stream));
-    return 0;
+    StreamScope ss(c, nullptr);
+    if (n) { if (int rc = h2d_segments(c, c->stage_a.p, up.data(), batch, ss.st)) return rc; }
+    if (int rc = poly_eval_on(c, c->stage_a.as<Fr>(), n, n, x, batch, c->small.as<Fr>(), ss.st)) return rc;
+    return d2h_one(c, out, c->small.p, sizeof(Fr) * batch, ss.st);
 }
 int b200_poly_eval(const b200_fr* coeffs, size_t n, const b200_fr* x, b200_fr* out) {
     const b200_fr* p[1] = {coeffs};
     return b200_poly_eval_batch(p, n, x, 1, out);
 }
-int b200_batch_invert_dev(void* d_a, size_t n, void* stream) {
-    B200_ENTER(c, d_a);
-    B200_CHECK(d_a, -1, "batch_invert: null pointer");
-    StreamScope ss(c, stream);
-    int rc = poly_batch_invert(reinterpret_cast<Fr*>(d_a), n, c->poly_ws, ss.st);
+static int batch_invert_on(Ctx* c, Fr* a, size_t n, cudaStream_t st) {
+    B200_CHECK(a, -1, "batch_invert: null pointer");
+    int rc = poly_batch_invert(a, n, c->poly_ws, st);
     if (!rc && n) g_launches += 1;
     return rc;
+}
+int b200_batch_invert_dev(void* d_a, size_t n, void* stream) {
+    B200_ENTER(c, d_a);
+    StreamScope ss(c, stream);
+    return batch_invert_on(c, reinterpret_cast<Fr*>(d_a), n, ss.st);
 }
 int b200_batch_invert(b200_fr* a, size_t n) {
     B200_ENTER(c, nullptr);
     B200_CHECK(a, -1, "batch_invert: null pointer");
     if (n == 0) return 0;
     if (c->stage_a.ensure(sizeof(Fr) * n)) return -2;
-    B200_CUDA(cudaMemcpyAsync(c->stage_a.p, a, sizeof(Fr) * n, cudaMemcpyHostToDevice, c->stream));
-    if (int rc = b200_batch_invert_dev(c->stage_a.p, n, nullptr)) return rc;
-    B200_CUDA(cudaMemcpyAsync(a, c->stage_a.p, sizeof(Fr) * n, cudaMemcpyDeviceToHost, c->stream));
-    B200_CUDA(cudaStreamSynchronize(c->stream));
-    return 0;
+    StreamScope ss(c, nullptr);
+    if (int rc = h2d_one(c, c->stage_a.p, a, sizeof(Fr) * n, ss.st)) return rc;
+    if (int rc = batch_invert_on(c, c->stage_a.as<Fr>(), n, ss.st)) return rc;
+    return d2h_one(c, a, c->stage_a.p, sizeof(Fr) * n, ss.st);
 }
-int b200_prefix_scan_dev(int product, const void* d_a, size_t n, const b200_fr* init, void* d_out, void* stream) {
-    B200_ENTER(c, d_a);
-    B200_CHECK(d_a && init && d_out, -1, "prefix_scan: null pointer");
-    const Fr iv = as_fr(init);
-    StreamScope ss(c, stream);
-    int rc = poly_prefix_scan(product != 0, reinterpret_cast<const Fr*>(d_a), n, n, &iv, reinterpret_cast<Fr*>(d_out), n, 1, c->poly_ws, ss.st);
-    if (!rc && n) g_launches += 3;
-    return rc;
-}
-int b200_prefix_scan_batch_dev(int product, const void* d_a, size_t a_stride, size_t n, size_t batch, const b200_fr* inits, void* d_out, size_t out_stride, void* stream) {
-    B200_ENTER(c, d_a);
-    B200_CHECK(d_a && inits && d_out, -1, "prefix_scan: null pointer");
+// `batch` columns: column p at a + p * a_stride, its running product / sum at out + p * out_stride, starting from inits[p]
+static int prefix_scan_on(Ctx* c, int product, const Fr* a, size_t a_stride, size_t n, size_t batch, const b200_fr* inits, Fr* out, size_t out_stride,
+                          cudaStream_t st) {
+    B200_CHECK(a && inits && out, -1, "prefix_scan: null pointer");
     B200_CHECK(batch <= 1 || (a_stride >= n && out_stride >= n), -1, "prefix_scan: column stride smaller than the column");
     if (batch == 0) return 0;
     std::vector<Fr> iv(batch);
     memcpy(iv.data(), inits, sizeof(Fr) * batch);
-    StreamScope ss(c, stream);
-    int rc = poly_prefix_scan(product != 0, reinterpret_cast<const Fr*>(d_a), a_stride, n, iv.data(), reinterpret_cast<Fr*>(d_out), out_stride, (int)batch, c->poly_ws, ss.st);
+    int rc = poly_prefix_scan(product != 0, a, a_stride, n, iv.data(), out, out_stride, (int)batch, c->poly_ws, st);
     if (!rc && n) g_launches += 3;
     return rc;
+}
+int b200_prefix_scan_dev(int product, const void* d_a, size_t n, const b200_fr* init, void* d_out, void* stream) {
+    B200_ENTER(c, d_a);
+    StreamScope ss(c, stream);
+    return prefix_scan_on(c, product, reinterpret_cast<const Fr*>(d_a), n, n, 1, init, reinterpret_cast<Fr*>(d_out), n, ss.st);
+}
+int b200_prefix_scan_batch_dev(int product, const void* d_a, size_t a_stride, size_t n, size_t batch, const b200_fr* inits, void* d_out, size_t out_stride, void* stream) {
+    B200_ENTER(c, d_a);
+    StreamScope ss(c, stream);
+    return prefix_scan_on(c, product, reinterpret_cast<const Fr*>(d_a), a_stride, n, batch, inits, reinterpret_cast<Fr*>(d_out), out_stride, ss.st);
 }
 int b200_prefix_scan(int product, const b200_fr* a, size_t n, const b200_fr* init, b200_fr* out) {
     B200_ENTER(c, nullptr);
     B200_CHECK(a && init && out, -1, "prefix_scan: null pointer");
     if (n == 0) return 0;
     if (c->stage_a.ensure(sizeof(Fr) * n) || c->stage_b.ensure(sizeof(Fr) * n)) return -2;
-    B200_CUDA(cudaMemcpyAsync(c->stage_a.p, a, sizeof(Fr) * n, cudaMemcpyHostToDevice, c->stream));
-    if (int rc = b200_prefix_scan_dev(product, c->stage_a.p, n, init, c->stage_b.p, nullptr)) return rc;
-    B200_CUDA(cudaMemcpyAsync(out, c->stage_b.p, sizeof(Fr) * n, cudaMemcpyDeviceToHost, c->stream));
-    B200_CUDA(cudaStreamSynchronize(c->stream));
-    return 0;
+    StreamScope ss(c, nullptr);
+    if (int rc = h2d_one(c, c->stage_a.p, a, sizeof(Fr) * n, ss.st)) return rc;
+    if (int rc = prefix_scan_on(c, product, c->stage_a.as<Fr>(), n, n, 1, init, c->stage_b.as<Fr>(), n, ss.st)) return rc;
+    return d2h_one(c, out, c->stage_b.p, sizeof(Fr) * n, ss.st);
+}
+static int kate_division_on(Ctx* c, const Fr* a, size_t n, const b200_fr* b, Fr* q, cudaStream_t st) {
+    B200_CHECK(a && b && q, -1, "kate_division: null pointer");
+    const Fr bv = as_fr(b);
+    int rc = poly_kate_division(a, n, &bv, q, c->poly_ws, st);
+    if (!rc && n > 1) g_launches += 3;
+    return rc;
 }
 int b200_kate_division_dev(const void* d_a, size_t n, const b200_fr* b, void* d_q, void* stream) {
     B200_ENTER(c, d_a);
-    B200_CHECK(d_a && b && d_q, -1, "kate_division: null pointer");
-    const Fr bv = as_fr(b);
     StreamScope ss(c, stream);
-    int rc = poly_kate_division(reinterpret_cast<const Fr*>(d_a), n, &bv, reinterpret_cast<Fr*>(d_q), c->poly_ws, ss.st);
-    if (!rc && n > 1) g_launches += 3;
-    return rc;
+    return kate_division_on(c, reinterpret_cast<const Fr*>(d_a), n, b, reinterpret_cast<Fr*>(d_q), ss.st);
 }
 int b200_kate_division(const b200_fr* a, size_t n, const b200_fr* b, b200_fr* q) {
     B200_ENTER(c, nullptr);
@@ -1141,62 +1180,63 @@ int b200_kate_division(const b200_fr* a, size_t n, const b200_fr* b, b200_fr* q)
     B200_CHECK(n >= 1, -1, "kate_division: empty polynomial");
     if (n == 1) return 0;
     if (c->stage_a.ensure(sizeof(Fr) * n) || c->stage_b.ensure(sizeof(Fr) * n)) return -2;
-    B200_CUDA(cudaMemcpyAsync(c->stage_a.p, a, sizeof(Fr) * n, cudaMemcpyHostToDevice, c->stream));
-    if (int rc = b200_kate_division_dev(c->stage_a.p, n, b, c->stage_b.p, nullptr)) return rc;
-    B200_CUDA(cudaMemcpyAsync(q, c->stage_b.p, sizeof(Fr) * (n - 1), cudaMemcpyDeviceToHost, c->stream));
-    B200_CUDA(cudaStreamSynchronize(c->stream));
-    return 0;
+    StreamScope ss(c, nullptr);
+    if (int rc = h2d_one(c, c->stage_a.p, a, sizeof(Fr) * n, ss.st)) return rc;
+    if (int rc = kate_division_on(c, c->stage_a.as<Fr>(), n, b, c->stage_b.as<Fr>(), ss.st)) return rc;
+    return d2h_one(c, q, c->stage_b.p, sizeof(Fr) * (n - 1), ss.st);
 }
 
 // ---- mv-lookup multiplicities --------------------------------------------------------------------------------------------------
-int b200_lookup_multiplicities_dev(const void* d_table, size_t n_table, const void* const* d_inputs, size_t n_inputs, size_t n_rows, void* d_m, uint64_t* missing, void* stream) {
-    B200_ENTER(c, d_table);
-    B200_CHECK(d_table && d_m && d_inputs && n_inputs >= 1, -1, "lookup_multiplicities: null pointer");
-    StreamScope ss(c, stream);
-    const void* d_ptrs = c->ring.push(d_inputs, sizeof(void*) * n_inputs, ss.st);
+// d_inputs: host array of device addresses
+static int lookup_on(Ctx* c, const Fr* table, size_t n_table, const void* const* d_inputs, size_t n_inputs, size_t n_rows, Fr* m, uint64_t* missing,
+                     cudaStream_t st) {
+    B200_CHECK(table && m && d_inputs && n_inputs >= 1, -1, "lookup_multiplicities: null pointer");
+    const void* d_ptrs = c->ring.push(d_inputs, sizeof(void*) * n_inputs, st);
     if (!d_ptrs) {
         if (c->small.ensure(sizeof(void*) * n_inputs)) return -2;
-        B200_CUDA(cudaMemcpyAsync(c->small.p, d_inputs, sizeof(void*) * n_inputs, cudaMemcpyHostToDevice, ss.st));
-        B200_CUDA(cudaStreamSynchronize(ss.st));
+        if (int rc = h2d_one(c, c->small.p, d_inputs, sizeof(void*) * n_inputs, st)) return rc;
+        B200_CUDA(cudaStreamSynchronize(st));
         d_ptrs = c->small.p;
     }
     unsigned long long* d_missing = nullptr;
-    if (int rc = lookup_multiplicities_run(reinterpret_cast<const Fr*>(d_table), n_table, reinterpret_cast<const Fr* const*>(d_ptrs), n_inputs, n_rows,
-                                           reinterpret_cast<Fr*>(d_m), c->msm_ws.misc, &d_missing, ss.st)) return rc;
+    if (int rc = lookup_multiplicities_run(table, n_table, reinterpret_cast<const Fr* const*>(d_ptrs), n_inputs, n_rows, m, c->msm_ws.misc, &d_missing, st)) return rc;
     g_launches += 3;
     if (missing) {
         unsigned long long h = 0;
-        B200_CUDA(cudaMemcpyAsync(&h, d_missing, sizeof h, cudaMemcpyDeviceToHost, ss.st));
-        B200_CUDA(cudaStreamSynchronize(ss.st));
+        if (int rc = d2h_one(c, &h, d_missing, sizeof h, st)) return rc;
         *missing = h;
     }
     return 0;
+}
+int b200_lookup_multiplicities_dev(const void* d_table, size_t n_table, const void* const* d_inputs, size_t n_inputs, size_t n_rows, void* d_m, uint64_t* missing, void* stream) {
+    B200_ENTER(c, d_table);
+    StreamScope ss(c, stream);
+    return lookup_on(c, reinterpret_cast<const Fr*>(d_table), n_table, d_inputs, n_inputs, n_rows, reinterpret_cast<Fr*>(d_m), missing, ss.st);
 }
 int b200_lookup_multiplicities(const b200_fr* table, size_t n_table, const b200_fr* const* inputs, size_t n_inputs, size_t n_rows, b200_fr* m, uint64_t* missing) {
     B200_ENTER(c, nullptr);
     B200_CHECK(table && inputs && m && n_inputs >= 1, -1, "lookup_multiplicities: null pointer");
     if (c->stage_a.ensure(sizeof(Fr) * (n_table + n_inputs * (n_rows ? n_rows : 1))) || c->stage_b.ensure(sizeof(Fr) * n_table)) return -2;
-    B200_CUDA(cudaMemcpyAsync(c->stage_a.p, table, sizeof(Fr) * n_table, cudaMemcpyHostToDevice, c->stream));
+    // the table, then every input column, back to back in stage_a
+    std::vector<HostSeg> up{HostSeg{(uint8_t*)const_cast<b200_fr*>(table), sizeof(Fr) * n_table}};
     std::vector<const void*> ptrs(n_inputs);
     for (size_t j = 0; j < n_inputs; ++j) {
         B200_CHECK(inputs[j] || n_rows == 0, -1, "lookup_multiplicities: inputs[%zu] is null", j);
         ptrs[j] = c->stage_a.as<Fr>() + n_table + j * n_rows;
-        if (n_rows) B200_CUDA(cudaMemcpyAsync(const_cast<void*>(ptrs[j]), inputs[j], sizeof(Fr) * n_rows, cudaMemcpyHostToDevice, c->stream));
+        if (n_rows) up.push_back(HostSeg{(uint8_t*)const_cast<b200_fr*>(inputs[j]), sizeof(Fr) * n_rows});
     }
-    uint64_t miss = 0;
-    if (int rc = b200_lookup_multiplicities_dev(c->stage_a.p, n_table, ptrs.data(), n_inputs, n_rows, c->stage_b.p, &miss, nullptr)) return rc;
-    B200_CUDA(cudaMemcpyAsync(m, c->stage_b.p, sizeof(Fr) * n_table, cudaMemcpyDeviceToHost, c->stream));
-    B200_CUDA(cudaStreamSynchronize(c->stream));
-    if (missing) *missing = miss;
-    return 0;
+    StreamScope ss(c, nullptr);
+    if (int rc = h2d_segments(c, c->stage_a.p, up.data(), up.size(), ss.st)) return rc;
+    if (int rc = lookup_on(c, c->stage_a.as<Fr>(), n_table, ptrs.data(), n_inputs, n_rows, c->stage_b.as<Fr>(), missing, ss.st)) return rc;
+    return d2h_one(c, m, c->stage_b.p, sizeof(Fr) * n_table, ss.st);
 }
 
 // ---- quotient numerator (evaluate_h) ------------------------------------------------------------------------------
 static_assert(sizeof(b200_instr) == sizeof(QInstr) && sizeof(b200_col_ref) == sizeof(QLoad), "ABI structs must match the kernel's");
-int b200_quotient_eval_dev(const void* const* d_columns, size_t n_columns, uint32_t k, uint32_t ext_k, const b200_col_ref* loads, size_t n_loads,
-                           const b200_fr* constants, size_t n_constants, const b200_instr* program, size_t n_instr, void* d_out, void* stream) {
-    B200_ENTER(c, d_out);
-    B200_CHECK(d_out && (n_columns == 0 || d_columns) && (n_loads == 0 || loads) && (n_constants == 0 || constants) && (n_instr == 0 || program), -1, "quotient_eval: null pointer");
+// columns: host array of device addresses
+static int quotient_eval_on(Ctx* c, const Fr* const* columns, size_t n_columns, uint32_t k, uint32_t ext_k, const b200_col_ref* loads, size_t n_loads,
+                            const b200_fr* constants, size_t n_constants, const b200_instr* program, size_t n_instr, Fr* out, cudaStream_t st) {
+    B200_CHECK(out && (n_columns == 0 || columns) && (n_loads == 0 || loads) && (n_constants == 0 || constants) && (n_instr == 0 || program), -1, "quotient_eval: null pointer");
     B200_CHECK(ext_k >= k && ext_k <= 28, -1, "quotient_eval: need k <= ext_k <= 28");
     const uint64_t N = 1ull << ext_k, scale = 1ull << (ext_k - k);
     std::vector<QLoad> ql(n_loads);
@@ -1205,11 +1245,17 @@ int b200_quotient_eval_dev(const void* const* d_columns, size_t n_columns, uint3
         const int64_t off = (int64_t)loads[i].rotation * (int64_t)scale;           // Rotation(r) on the extended domain = r * 2^(ext_k - k)
         ql[i].offset = (uint32_t)(((off % (int64_t)N) + (int64_t)N) % (int64_t)N);
     }
-    StreamScope ss(c, stream);
-    int rc = quotient_eval_run(reinterpret_cast<const Fr* const*>(d_columns), n_columns, ext_k, ql.data(), n_loads, reinterpret_cast<const Fr*>(constants), n_constants,
-                               reinterpret_cast<const QInstr*>(program), n_instr, reinterpret_cast<Fr*>(d_out), c->quot_ws, ss.st);
+    int rc = quotient_eval_run(columns, n_columns, ext_k, ql.data(), n_loads, reinterpret_cast<const Fr*>(constants), n_constants,
+                               reinterpret_cast<const QInstr*>(program), n_instr, out, c->quot_ws, st);
     if (!rc) g_launches += 1;
     return rc;
+}
+int b200_quotient_eval_dev(const void* const* d_columns, size_t n_columns, uint32_t k, uint32_t ext_k, const b200_col_ref* loads, size_t n_loads,
+                           const b200_fr* constants, size_t n_constants, const b200_instr* program, size_t n_instr, void* d_out, void* stream) {
+    B200_ENTER(c, d_out);
+    StreamScope ss(c, stream);
+    return quotient_eval_on(c, reinterpret_cast<const Fr* const*>(d_columns), n_columns, k, ext_k, loads, n_loads, constants, n_constants, program, n_instr,
+                            reinterpret_cast<Fr*>(d_out), ss.st);
 }
 int b200_quotient_eval(const b200_fr* const* columns, size_t n_columns, uint32_t k, uint32_t ext_k, const b200_col_ref* loads, size_t n_loads,
                        const b200_fr* constants, size_t n_constants, const b200_instr* program, size_t n_instr, b200_fr* out) {
@@ -1218,16 +1264,17 @@ int b200_quotient_eval(const b200_fr* const* columns, size_t n_columns, uint32_t
     B200_CHECK(ext_k >= 1 && ext_k <= 28, -1, "quotient_eval: ext_k out of range");
     const size_t N = (size_t)1 << ext_k;
     if (c->stage_a.ensure(sizeof(Fr) * N * (n_columns ? n_columns : 1)) || c->stage_b.ensure(sizeof(Fr) * N)) return -2;
-    std::vector<const void*> ptrs(n_columns);
+    std::vector<const Fr*> ptrs(n_columns);
     std::vector<HostSeg> up(n_columns);
     for (size_t i = 0; i < n_columns; ++i) {
         B200_CHECK(columns[i], -1, "quotient_eval: column %zu is null", i);
         ptrs[i] = c->stage_a.as<Fr>() + i * N;
         up[i] = HostSeg{(uint8_t*)const_cast<b200_fr*>(columns[i]), sizeof(Fr) * N};
     }
-    if (int rc = h2d_segments(c, c->stage_a.p, up.data(), n_columns, c->stream)) return rc;
-    if (int rc = b200_quotient_eval_dev(ptrs.data(), n_columns, k, ext_k, loads, n_loads, constants, n_constants, program, n_instr, c->stage_b.p, nullptr)) return rc;
-    return d2h_one(c, out, c->stage_b.p, sizeof(Fr) * N, c->stream);
+    StreamScope ss(c, nullptr);
+    if (int rc = h2d_segments(c, c->stage_a.p, up.data(), n_columns, ss.st)) return rc;
+    if (int rc = quotient_eval_on(c, ptrs.data(), n_columns, k, ext_k, loads, n_loads, constants, n_constants, program, n_instr, c->stage_b.as<Fr>(), ss.st)) return rc;
+    return d2h_one(c, out, c->stage_b.p, sizeof(Fr) * N, ss.st);
 }
 
 // evaluate_h at its natural boundary: the CPU evaluator receives coefficient-form polynomials and builds their cosets itself
@@ -1255,8 +1302,8 @@ int b200_evaluate_h(const b200_fr* const* polys, const size_t* lengths, size_t n
     if (c->stage_a.ensure(sizeof(Fr) * (max_len ? max_len : 1) * sub) || c->stage_b.ensure(sizeof(Fr) * N * sub)) return -2;
     StreamScope ss(c, nullptr);
     Fr* ext = c->stage_c.as<Fr>();
-    NttScale pre, none;
-    pre.mode = 3; pre.c[0] = fp_one<FrTag>(); pre.c[1] = as_fr(zeta); pre.c[2] = as_fr(zeta) * as_fr(zeta);
+    const NttScale pre = coset_scale(as_fr(zeta));
+    NttScale none;
     std::vector<size_t> group;           // coefficient columns of equal length are transformed together
     auto flush = [&](size_t len) -> int {
         if (group.empty()) return 0;
@@ -1284,15 +1331,13 @@ int b200_evaluate_h(const b200_fr* const* polys, const size_t* lengths, size_t n
         group.push_back(i);
     }
     if (int rc = flush(cur_len)) return rc;
-    std::vector<const void*> ptrs(n_columns);
+    std::vector<const Fr*> ptrs(n_columns);
     for (size_t i = 0; i < n_columns; ++i) ptrs[i] = ext + i * N;
     Fr* h = c->stage_b.as<Fr>();
-    if (int rc = b200_quotient_eval_dev(ptrs.data(), n_columns, k, ext_k, loads, n_loads, constants, n_constants, program, n_instr, h, ss.st)) return rc;
+    if (int rc = quotient_eval_on(c, ptrs.data(), n_columns, k, ext_k, loads, n_loads, constants, n_constants, program, n_instr, h, ss.st)) return rc;
     if (t_evaluations) {
-        if (int rc = b200_poly_scale_cycle_dev(h, N, t_evaluations, t_period, ss.st)) return rc;
-        NttScale post;
-        const Fr z = as_fr(zeta), z2 = z * z, d = as_fr(ext_ifft_divisor);
-        post.mode = 3; post.c[0] = d; post.c[1] = d * z2; post.c[2] = d * z;
+        if (int rc = scale_cycle_on(c, h, N, t_evaluations, t_period, ss.st)) return rc;
+        const NttScale post = coset_unscale(as_fr(zeta), as_fr(ext_ifft_divisor));
         if (int rc = ntt_call(c, h, N, N, ext, h, N, ext_k, as_fr(ext_omega_inv), none, post, 1, ss.st)) return rc;      // `ext` is free again: scratch
     }
     return d2h_one(c, out, h, sizeof(Fr) * N, ss.st);

@@ -271,7 +271,7 @@ def test_msm_k17_and_linearity_k20():
 
 
 # ---- polynomial ops ----------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("n", [1, 7, 4096, 4097, 100000, 1 << 17])
+@pytest.mark.parametrize("n", [1, 7, 4096, 4097, 100000, 1 << 17, (1 << 19) + 3])      # the last moves through the 16 MiB bounce chunks
 def test_poly_ops_vs_oracle(n):
     a, b = orc.gen_scalars(n, seed=n), orc.gen_scalars(n, seed=n + 1)
     s = orc.gen_scalars(1, seed=n + 2)[0]
@@ -387,7 +387,7 @@ def test_empty_and_tiny_inputs():
     out = np.zeros(12, np.uint64)
     nat.check(L.b200_msm(C.c_uint64(bases.handle), nat.ptr(np.zeros((1, 4), np.uint64)), C.c_size_t(0), nat.ptr(out)))     # n = 0 -> identity
     assert np.array_equal(out, np.array([0] * 4 + list(H.fq_wire(1)) + [0] * 4, np.uint64))
-    nat.check(L.b200_msm_batch(C.c_uint64(bases.handle), None, C.c_size_t(8), C.c_size_t(0), nat.ptr(out)) if False else 0)
+    assert L.b200_msm_batch(C.c_uint64(bases.handle), None, C.c_size_t(8), C.c_size_t(0), nat.ptr(out)) == -1      # NULL columns, even for batch 0
     assert h2.best_multiexp_batch([], bases).shape == (0, 12)
     one = orc.gen_scalars(1, seed=1)
     assert np.array_equal(jac_to_affine(h2.best_multiexp(one, bases))[0], orc.msm(one, bases_np[:1], 1))
