@@ -15,6 +15,7 @@
 #include <vector>
 
 #include "../../include/ezkl_b200.h"
+#include "../../include/ezkl_b200_parts.h"
 #include "msm.cuh"
 #include "ntt.cuh"
 #include "poly.cuh"
@@ -294,6 +295,37 @@ static int d2h_segments(Ctx* c, const void* d_src, const HostSeg* segs, size_t n
             B200_CUDA(cudaEventSynchronize(c->bounce_ev[(i - 1) & 1]));
             seg_copy_parallel(segs, nsegs, off, off + nb, c->bounce[(i - 1) & 1], false);
         }
+    }
+    return 0;
+}
+// every stride-th element of one caller buffer (count elements of `elem` bytes) -> contiguous device range, through the same pinned
+// bounce buffers and pipeline as h2d_segments (a coset part of an extended column).  When the call returns every source element has been read.
+static void gather_range(const uint8_t* src, size_t i0, size_t i1, size_t elem, size_t stride_bytes, uint8_t* flat) {
+    for (size_t i = i0; i < i1; ++i) memcpy(flat + i * elem, src + i * stride_bytes, elem);
+}
+static int h2d_strided(Ctx* c, void* d_dst, const uint8_t* src, size_t count, size_t elem, size_t stride, cudaStream_t st) {
+    if (int rc = bounce_ready(c)) return rc;
+    const size_t per = BOUNCE_BYTES / elem, stride_bytes = stride * elem;
+    int slot = 0;
+    for (size_t i0 = 0; i0 < count; i0 += per, slot ^= 1) {
+        const size_t m = count - i0 < per ? count - i0 : per;
+        B200_CUDA(cudaEventSynchronize(c->bounce_ev[slot]));                       // the DMA that last read this slot is done
+        const uint8_t* s0 = src + i0 * stride_bytes;
+        uint8_t* flat = c->bounce[slot];
+        const int T = 4;
+        if (m * elem < ((size_t)2 << 20)) gather_range(s0, 0, m, elem, stride_bytes, flat);
+        else {
+            std::thread th[T - 1];
+            const size_t q = (m + T - 1) / T;
+            for (int t = 1; t < T; ++t) {
+                const size_t a = q * t, b = a + q < m ? a + q : m;
+                if (a < b) th[t - 1] = std::thread([=] { gather_range(s0, a, b, elem, stride_bytes, flat); });
+            }
+            gather_range(s0, 0, q < m ? q : m, elem, stride_bytes, flat);
+            for (int t = 1; t < T; ++t) if (th[t - 1].joinable()) th[t - 1].join();
+        }
+        B200_CUDA(cudaMemcpyAsync((uint8_t*)d_dst + i0 * elem, flat, m * elem, cudaMemcpyHostToDevice, st));
+        B200_CUDA(cudaEventRecord(c->bounce_ev[slot], st));
     }
     return 0;
 }
@@ -1340,6 +1372,220 @@ int b200_evaluate_h(const b200_fr* const* polys, const size_t* lengths, size_t n
         const NttScale post = coset_unscale(as_fr(zeta), as_fr(ext_ifft_divisor));
         if (int rc = ntt_call(c, h, N, N, ext, h, N, ext_k, as_fr(ext_omega_inv), none, post, 1, ss.st)) return rc;      // `ext` is free again: scratch
     }
+    return d2h_one(c, out, h, sizeof(Fr) * N, ss.st);
+}
+
+// ---- the extended domain one coset part at a time (include/ezkl_b200_parts.h) ---------------------------------------------------------
+// Power tables of the parts' pre-scales c_r^i (c_r = zeta * ext_omega^r, i < 2^k) for r in [part0, part0 + nparts), built on the host and
+// staged into c->small; part_scale(r - part0) selects one.
+static int stage_part_tables(Ctx* c, uint32_t k, uint32_t part0, uint32_t nparts, const Fr& ext_omega, const Fr& zeta, cudaStream_t st) {
+    const size_t len = geo_table_len(k);
+    std::vector<Fr> h(len * nparts);
+    Fr cr = zeta * fp_pow_u64(ext_omega, part0);
+    for (uint32_t j = 0; j < nparts; ++j) { geo_table_fill(cr, k, h.data() + len * j); cr = cr * ext_omega; }
+    if (c->small.ensure(sizeof(Fr) * h.size())) return -2;
+    return h2d_one(c, c->small.p, h.data(), sizeof(Fr) * h.size(), st);
+}
+static NttScale part_scale(Ctx* c, uint32_t k, uint32_t j) {
+    NttScale s;
+    s.mode = NTT_SCALE_GEOMETRIC;
+    s.lo_bits = geo_lo_bits(k);
+    s.lo = c->small.as<Fr>() + geo_table_len(k) * j;
+    s.hi = s.lo + ((size_t)1 << s.lo_bits);
+    return s;
+}
+static int part_args_check(uint32_t k, uint32_t ext_k, uint32_t part, size_t n_coeffs) {
+    B200_CHECK(k >= 1 && ext_k >= k && ext_k <= 28, -1, "coeff_to_extended_part: need 1 <= k <= ext_k <= 28");
+    B200_CHECK(part < (1u << (ext_k - k)), -1, "coeff_to_extended_part: part %u >= 2^(ext_k - k)", part);
+    B200_CHECK(n_coeffs <= ((size_t)1 << k), -1, "coeff_to_extended_part: %zu coefficients > 2^k", n_coeffs);
+    return 0;
+}
+int b200_coeff_to_extended_part_dev(const void* d_coeffs, size_t src_stride, size_t n_coeffs, void* d_tmp, void* d_out, size_t dst_stride, uint32_t k,
+                                    uint32_t ext_k, uint32_t part, const b200_fr* ext_omega, const b200_fr* zeta, size_t batch, void* stream) {
+    B200_ENTER(c, d_coeffs);
+    B200_CHECK(d_coeffs && d_tmp && d_out && ext_omega && zeta, -1, "coeff_to_extended_part: null pointer");
+    if (int rc = part_args_check(k, ext_k, part, n_coeffs)) return rc;
+    B200_CHECK(batch <= 65535, -1, "coeff_to_extended_part: batch %zu out of range", batch);
+    if (batch == 0) return 0;
+    StreamScope ss(c, stream);
+    const Fr w = as_fr(ext_omega);
+    if (int rc = stage_part_tables(c, k, part, 1, w, as_fr(zeta), ss.st)) return rc;
+    NttScale none;
+    return ntt_call(c, reinterpret_cast<const Fr*>(d_coeffs), src_stride, n_coeffs, reinterpret_cast<Fr*>(d_tmp), reinterpret_cast<Fr*>(d_out), dst_stride, k,
+                    fp_pow_u64(w, 1ull << (ext_k - k)), part_scale(c, k, 0), none, (int)batch, ss.st);
+}
+int b200_coeff_to_extended_part_batch(const b200_fr* const* coeffs, size_t batch, size_t n_coeffs, uint32_t k, uint32_t ext_k, uint32_t part,
+                                      const b200_fr* ext_omega, const b200_fr* zeta, b200_fr* const* out) {
+    B200_ENTER(c, nullptr);
+    B200_CHECK(coeffs && out && ext_omega && zeta, -1, "coeff_to_extended_part: null pointer");
+    if (int rc = part_args_check(k, ext_k, part, n_coeffs)) return rc;
+    if (batch == 0) return 0;
+    const size_t n = (size_t)1 << k, n_in = n_coeffs ? n_coeffs : 1;
+    size_t sub = call_budget() / (sizeof(Fr) * n * 3);
+    if (sub < 1) sub = 1;
+    if (sub > batch) sub = batch;
+    if (sub > 65535) sub = 65535;
+    if (c->stage_a.ensure(sizeof(Fr) * n_in * sub) || c->stage_b.ensure(sizeof(Fr) * n * sub) || c->stage_c.ensure(sizeof(Fr) * n * sub)) return -2;
+    StreamScope ss(c, nullptr);
+    const Fr w = as_fr(ext_omega);
+    if (int rc = stage_part_tables(c, k, part, 1, w, as_fr(zeta), ss.st)) return rc;
+    const Fr wn = fp_pow_u64(w, 1ull << (ext_k - k));
+    NttScale none;
+    for (size_t b0 = 0; b0 < batch; b0 += sub) {
+        const size_t nb = batch - b0 < sub ? batch - b0 : sub;
+        std::vector<HostSeg> up(nb), down(nb);
+        for (size_t p = 0; p < nb; ++p) {
+            B200_CHECK((coeffs[b0 + p] || n_coeffs == 0) && out[b0 + p], -1, "coeff_to_extended_part: polynomial %zu is null", b0 + p);
+            up[p] = HostSeg{(uint8_t*)const_cast<b200_fr*>(coeffs[b0 + p]), sizeof(Fr) * n_coeffs};
+            down[p] = HostSeg{(uint8_t*)out[b0 + p], sizeof(Fr) * n};
+        }
+        if (n_coeffs) { if (int rc = h2d_segments(c, c->stage_a.p, up.data(), nb, ss.st)) return rc; }
+        if (int rc = ntt_call(c, c->stage_a.as<Fr>(), n_in, n_coeffs, c->stage_b.as<Fr>(), c->stage_c.as<Fr>(), n, k, wn, part_scale(c, k, 0), none, (int)nb, ss.st)) return rc;
+        if (int rc = d2h_segments(c, c->stage_c.p, down.data(), nb, ss.st)) return rc;
+    }
+    return 0;
+}
+
+// argument checks shared by both evaluate_h_parts entries; counts the coefficient and extended columns
+static int parts_args_check(const size_t* lengths, size_t n_columns, uint32_t k, uint32_t ext_k, const b200_fr* t_evaluations, uint32_t t_period,
+                            const b200_fr* ext_omega_inv, const b200_fr* ext_ifft_divisor, size_t* n_coeff, size_t* n_ext, size_t* coeff_elems) {
+    B200_CHECK(k >= 1 && ext_k >= k && ext_k <= 28, -1, "evaluate_h_parts: need 1 <= k <= ext_k <= 28");
+    const uint32_t d = 1u << (ext_k - k);
+    B200_CHECK(!t_evaluations || (t_period >= 1 && t_period <= 1024 && d % t_period == 0 && ext_omega_inv && ext_ifft_divisor), -1,
+               "evaluate_h_parts: finishing needs t_evaluations, a period dividing 2^(ext_k - k) and the inverse-transform constants");
+    const size_t n = (size_t)1 << k, N = (size_t)1 << ext_k;
+    *n_coeff = *n_ext = *coeff_elems = 0;
+    for (size_t i = 0; i < n_columns; ++i) {
+        if (lengths[i] == N) ++*n_ext;
+        else {
+            B200_CHECK(lengths[i] >= 1 && lengths[i] <= n, -1, "evaluate_h_parts: column %zu has %zu elements: neither <= 2^k (coefficients) nor 2^ext_k (extended)", i, lengths[i]);
+            ++*n_coeff; *coeff_elems += lengths[i];
+        }
+    }
+    return 0;
+}
+// The d parts of one evaluate_h.  Column i is a coefficient column (coeff[i], device, lengths[i] <= 2^k), or an extended column read either in
+// place (ext_dev[i], device, 2^ext_k elements, stride d per part) or gathered from the host per part (ext_host[i]).  parts: device buffer of
+// (n_coeff + n_ext_host) * 2^k elements; scratch: 2^ext_k elements; out: 2^ext_k elements.  Tables of the pre-scales are in c->small.
+static int evaluate_h_parts_on(Ctx* c, const Fr* const* coeff, const Fr* const* ext_dev, const b200_fr* const* ext_host, const size_t* lengths, size_t n_columns,
+                               uint32_t k, uint32_t ext_k, const Fr& ext_omega, const Fr& zeta, const b200_col_ref* loads, size_t n_loads,
+                               const b200_fr* constants, size_t n_constants, const b200_instr* program, size_t n_instr, const b200_fr* t_evaluations,
+                               uint32_t t_period, const b200_fr* ext_omega_inv, const b200_fr* ext_ifft_divisor, Fr* parts, Fr* scratch, Fr* out, cudaStream_t st) {
+    const uint32_t log_d = ext_k - k, d = 1u << log_d;
+    const size_t n = (size_t)1 << k, N = (size_t)1 << ext_k;
+    const Fr wn = fp_pow_u64(ext_omega, d);
+    if (int rc = stage_part_tables(c, k, 0, d, ext_omega, zeta, st)) return rc;
+    // every column's buffer inside a part: coefficient columns, then host-gathered extended columns, in column order
+    std::vector<size_t> slot(n_columns, 0);
+    size_t ns = 0;
+    for (size_t i = 0; i < n_columns; ++i) if (lengths[i] != N) slot[i] = ns++;
+    for (size_t i = 0; i < n_columns; ++i) if (lengths[i] == N && ext_host) slot[i] = ns++;
+    // runs of coefficient columns transformed in one launch: equal length, sources at one stride, consecutive slots, at most d columns
+    // (the transform scratch holds d parts)
+    struct Run { size_t first, last, count, stride; };
+    std::vector<Run> runs;
+    for (size_t i = 0; i < n_columns; ++i) {
+        if (lengths[i] == N) continue;
+        if (!runs.empty()) {
+            Run& r = runs.back();
+            const uintptr_t a = (uintptr_t)coeff[r.last], b = (uintptr_t)coeff[i];
+            const size_t gap = b > a ? (size_t)(b - a) / sizeof(Fr) : 0;
+            if (lengths[i] == lengths[r.first] && b > a && (b - a) % sizeof(Fr) == 0 && gap >= lengths[i] && (r.count == 1 || gap == r.stride) && r.count < d) {
+                r.stride = gap; r.last = i; ++r.count; continue;
+            }
+        }
+        runs.push_back(Run{i, i, 1, lengths[i]});
+    }
+    // per-part program: the caller's, then (finishing) one multiplication of the row result by the part's vanishing factor
+    std::vector<QInstr> prog(n_instr);
+    if (n_instr) memcpy(prog.data(), program, sizeof(QInstr) * n_instr);
+    std::vector<Fr> consts(n_constants);
+    if (n_constants) memcpy(consts.data(), constants, sizeof(Fr) * n_constants);
+    const bool fuse = t_evaluations && n_instr;
+    if (fuse) {
+        QInstr m;
+        m.op_dst = QOP_MUL | Q_NOSTORE; m.a = (uint32_t)QSRC_PREV << 30; m.b = ((uint32_t)QSRC_CONST << 30) | (uint32_t)n_constants; m.c = 0;
+        prog.push_back(m);
+        consts.push_back(fp_zero<FrTag>());
+    }
+    std::vector<QLoad> ql(n_loads);
+    for (size_t i = 0; i < n_loads; ++i) {
+        ql[i].column = loads[i].column;
+        ql[i].offset = (uint32_t)((((int64_t)loads[i].rotation % (int64_t)n) + (int64_t)n) % (int64_t)n);     // Rotation(rot) inside a part
+    }
+    std::vector<const Fr*> ptrs(n_columns);
+    std::vector<uint32_t> shift(n_columns);
+    NttScale none;
+    for (uint32_t r = 0; r < d; ++r) {
+        const NttScale pre = part_scale(c, k, r);
+        for (const Run& run : runs) {
+            if (int rc = ntt_call(c, coeff[run.first], run.stride, lengths[run.first], scratch, parts + slot[run.first] * n, n, k, wn, pre, none, (int)run.count, st)) return rc;
+        }
+        for (size_t i = 0; i < n_columns; ++i) {
+            if (lengths[i] != N) { ptrs[i] = parts + slot[i] * n; shift[i] = 0; }
+            else if (ext_host) {
+                B200_CHECK(ext_host[i], -1, "evaluate_h_parts: column %zu is null", i);
+                if (int rc = h2d_strided(c, parts + slot[i] * n, reinterpret_cast<const uint8_t*>(ext_host[i] + r), n, sizeof(Fr), d, st)) return rc;
+                ptrs[i] = parts + slot[i] * n; shift[i] = 0;
+            } else { ptrs[i] = ext_dev[i] + r; shift[i] = log_d; }
+        }
+        if (fuse) consts.back() = as_fr(t_evaluations + (r % t_period));
+        if (int rc = quotient_eval_part_run(ptrs.data(), shift.data(), n_columns, k, log_d, ql.data(), n_loads, consts.data(), consts.size(), prog.data(), prog.size(),
+                                            out + r, c->quot_ws, st)) return rc;
+        g_launches += 1;
+    }
+    if (t_evaluations) {
+        const NttScale post = coset_unscale(zeta, as_fr(ext_ifft_divisor));
+        if (int rc = ntt_call(c, out, N, N, scratch, out, N, ext_k, as_fr(ext_omega_inv), none, post, 1, st)) return rc;
+    }
+    return 0;
+}
+int b200_evaluate_h_parts_dev(const void* const* d_polys, const size_t* lengths, size_t n_columns, uint32_t k, uint32_t ext_k, const b200_fr* ext_omega,
+                              const b200_fr* zeta, const b200_col_ref* loads, size_t n_loads, const b200_fr* constants, size_t n_constants,
+                              const b200_instr* program, size_t n_instr, const b200_fr* t_evaluations, uint32_t t_period, const b200_fr* ext_omega_inv,
+                              const b200_fr* ext_ifft_divisor, void* d_out, void* stream) {
+    B200_ENTER(c, d_out);
+    B200_CHECK(d_out && ext_omega && zeta && (n_columns == 0 || (d_polys && lengths)) && (n_loads == 0 || loads) && (n_constants == 0 || constants) &&
+               (n_instr == 0 || program), -1, "evaluate_h_parts: null pointer");
+    size_t n_coeff, n_ext, coeff_elems;
+    if (int rc = parts_args_check(lengths, n_columns, k, ext_k, t_evaluations, t_period, ext_omega_inv, ext_ifft_divisor, &n_coeff, &n_ext, &coeff_elems)) return rc;
+    std::vector<const Fr*> cols(n_columns);
+    for (size_t i = 0; i < n_columns; ++i) { B200_CHECK(d_polys[i], -1, "evaluate_h_parts: column %zu is null", i); cols[i] = reinterpret_cast<const Fr*>(d_polys[i]); }
+    const size_t n = (size_t)1 << k, N = (size_t)1 << ext_k;
+    if (c->stage_c.ensure(sizeof(Fr) * n * (n_coeff ? n_coeff : 1)) || c->stage_b.ensure(sizeof(Fr) * N)) return -2;
+    StreamScope ss(c, stream);
+    return evaluate_h_parts_on(c, cols.data(), cols.data(), nullptr, lengths, n_columns, k, ext_k, as_fr(ext_omega), as_fr(zeta), loads, n_loads, constants, n_constants,
+                               program, n_instr, t_evaluations, t_period, ext_omega_inv, ext_ifft_divisor, c->stage_c.as<Fr>(), c->stage_b.as<Fr>(),
+                               reinterpret_cast<Fr*>(d_out), ss.st);
+}
+int b200_evaluate_h_parts(const b200_fr* const* polys, const size_t* lengths, size_t n_columns, uint32_t k, uint32_t ext_k, const b200_fr* ext_omega,
+                          const b200_fr* zeta, const b200_col_ref* loads, size_t n_loads, const b200_fr* constants, size_t n_constants,
+                          const b200_instr* program, size_t n_instr, const b200_fr* t_evaluations, uint32_t t_period, const b200_fr* ext_omega_inv,
+                          const b200_fr* ext_ifft_divisor, b200_fr* out) {
+    B200_ENTER(c, nullptr);
+    B200_CHECK(out && ext_omega && zeta && (n_columns == 0 || (polys && lengths)) && (n_loads == 0 || loads) && (n_constants == 0 || constants) &&
+               (n_instr == 0 || program), -1, "evaluate_h_parts: null pointer");
+    size_t n_coeff, n_ext, coeff_elems;
+    if (int rc = parts_args_check(lengths, n_columns, k, ext_k, t_evaluations, t_period, ext_omega_inv, ext_ifft_divisor, &n_coeff, &n_ext, &coeff_elems)) return rc;
+    for (size_t i = 0; i < n_columns; ++i) B200_CHECK(polys[i], -1, "evaluate_h_parts: column %zu is null", i);
+    const size_t n = (size_t)1 << k, N = (size_t)1 << ext_k;
+    // device layout: stage_a = resident coefficients (packed in column order), stage_c = one part of every column, stage_b = [output | scratch]
+    if (c->stage_a.ensure(sizeof(Fr) * (coeff_elems ? coeff_elems : 1)) || c->stage_c.ensure(sizeof(Fr) * n * (n_coeff + n_ext ? n_coeff + n_ext : 1)) ||
+        c->stage_b.ensure(sizeof(Fr) * N * 2)) return -2;
+    std::vector<const Fr*> cols(n_columns, nullptr);
+    std::vector<HostSeg> up;
+    size_t off = 0;
+    for (size_t i = 0; i < n_columns; ++i) {
+        if (lengths[i] == N) continue;
+        cols[i] = c->stage_a.as<Fr>() + off;
+        up.push_back(HostSeg{(uint8_t*)const_cast<b200_fr*>(polys[i]), sizeof(Fr) * lengths[i]});
+        off += lengths[i];
+    }
+    StreamScope ss(c, nullptr);
+    if (!up.empty()) { if (int rc = h2d_segments(c, c->stage_a.p, up.data(), up.size(), ss.st)) return rc; }
+    Fr* h = c->stage_b.as<Fr>();
+    if (int rc = evaluate_h_parts_on(c, cols.data(), nullptr, polys, lengths, n_columns, k, ext_k, as_fr(ext_omega), as_fr(zeta), loads, n_loads, constants, n_constants,
+                                     program, n_instr, t_evaluations, t_period, ext_omega_inv, ext_ifft_divisor, c->stage_c.as<Fr>(), h + N, h, ss.st)) return rc;
     return d2h_one(c, out, h, sizeof(Fr) * N, ss.st);
 }
 

@@ -13,9 +13,10 @@
 //     per-stage twiddle table is staged into shared memory with cp.async.bulk (TMA) + mbarrier.
 //   k_ntt_pass (v1): one radix-2 stage per shared-memory round trip; kept for tiny passes and as B200_NTT_V=1.
 // Coset pre-scaling (zeta^(i mod 3)), zero padding and the 1/N (and zeta^-(i mod 3)) post-scaling of the extended-domain
-// transforms are fused into the first load / last store.  Algorithmic HBM traffic: 64 B per element per transform; this
-// schedule moves 64 B per element per PASS (2 passes up to 2^20, 3 above).  The kernels are bound by the 254-bit multiply
-// (10-15 per element), not by HBM: see DESIGN.md §4.3.
+// transforms are fused into the first load / last store, and so is the geometric pre-scale c^i of a coset-part transform
+// (coeff_to_extended_part: c = zeta * ext_omega^r, from two host-built power tables; a separate kernel instantiation).
+// Algorithmic HBM traffic: 64 B per element per transform; this schedule moves 64 B per element per PASS (2 passes up to
+// 2^20, 3 above).  The kernels are bound by the 254-bit multiply (10-15 per element), not by HBM: see DESIGN.md §4.3.
 #include <cstdlib>
 #include "ntt.cuh"
 
@@ -53,6 +54,13 @@ DEV void sh_put(uint4* lo, uint4* hi, uint32_t i, const Fr& v) {
     hi[i] = make_uint4(v.l[4], v.l[5], v.l[6], v.l[7]);
 }
 
+// c^idx of the geometric pre-scale: two table loads, one multiplication
+DEV Fr geo_power(const NttScale& s, uint64_t idx) {
+    return fp_load(s.lo + (idx & ((1ull << s.lo_bits) - 1))) * fp_load(s.hi + (idx >> s.lo_bits));
+}
+
+// GEO: the first load applies NTT_SCALE_GEOMETRIC; a separate instantiation, so the other modes keep their code unchanged
+template <bool GEO>
 __global__ void __launch_bounds__(1024, 1) k_ntt_pass(const PassArgs a) {
     extern __shared__ uint4 sh[];
     const uint32_t M = 1u << a.logm, G = 1u << a.log_g, total = M << a.log_g;
@@ -75,7 +83,8 @@ __global__ void __launch_bounds__(1024, 1) k_ntt_pass(const PassArgs a) {
         if (idx < a.n_in) {
             v = fp_load(src + idx);
             if (a.first) {
-                if (a.pre.mode == 1) v = v * a.pre.c[0];
+                if constexpr (GEO) v = v * geo_power(a.pre, idx);
+                else if (a.pre.mode == 1) v = v * a.pre.c[0];
                 else if (a.pre.mode == 3) { uint32_t m3 = (uint32_t)(idx % 3); if (m3) v = v * a.pre.c[m3]; }
             }
         }
@@ -146,6 +155,7 @@ DEV void mbar_wait(uint64_t* bar, uint32_t phase) {
                  ::"r"(smem_u32(bar)), "r"(phase) : "memory");
 }
 
+template <bool GEO>
 __global__ void __launch_bounds__(256, 3) k_ntt_pass2(const PassArgs a) {
     extern __shared__ uint4 sh[];
     __shared__ uint64_t bar;
@@ -192,7 +202,8 @@ __global__ void __launch_bounds__(256, 3) k_ntt_pass2(const PassArgs a) {
                 if (idx < a.n_in) {
                     x[j] = fp_load(a.peer_on ? a.src_peers[idx >> a.log_slice] + (idx & slice_mask) : src + idx);
                     if (a.first) {
-                        if (a.pre.mode == 1) x[j] = x[j] * a.pre.c[0];
+                        if constexpr (GEO) x[j] = x[j] * geo_power(a.pre, idx);
+                        else if (a.pre.mode == 1) x[j] = x[j] * a.pre.c[0];
                         else if (a.pre.mode == 3) { uint32_t m3 = (uint32_t)(idx % 3); if (m3) x[j] = x[j] * a.pre.c[m3]; }
                     }
                 }
@@ -295,6 +306,17 @@ static void choose_passes(uint32_t log_n, int* npass, int logm[3]) {
 }
 int ntt_launches_per_run(uint32_t log_n) { int np, lm[3]; choose_passes(log_n, &np, lm); return np; }
 
+uint32_t geo_lo_bits(uint32_t log_n) { return (log_n + 1) / 2; }
+size_t geo_table_len(uint32_t log_n) { return ((size_t)1 << geo_lo_bits(log_n)) + ((size_t)1 << (log_n - geo_lo_bits(log_n))); }
+void geo_table_fill(const Fr& c, uint32_t log_n, Fr* out) {
+    const uint32_t b = geo_lo_bits(log_n);
+    const size_t nlo = (size_t)1 << b, nhi = (size_t)1 << (log_n - b);
+    Fr v = fp_one<FrTag>();
+    for (size_t i = 0; i < nlo; ++i) { out[i] = v; v = v * c; }          // v = c^(2^b) on exit
+    Fr w = fp_one<FrTag>();
+    for (size_t i = 0; i < nhi; ++i) { out[nlo + i] = w; w = w * v; }
+}
+
 static Fr host_pow(const Fr& b, uint64_t e) { return fp_pow_u64(b, e); }
 
 NttPlan* NttContext::get(uint32_t log_n, const Fr& omega, cudaStream_t st) {
@@ -360,9 +382,10 @@ static int launch_pass(PassArgs& a, uint64_t lines, int batch, cudaStream_t st) 
     uint32_t threads; size_t smem;
     if (!plan_pass_v2(a, lines, batch, &threads, &smem)) return launch_pass_v1(a, lines, batch, st);
     B200_CHECK(threads <= 256 && smem <= 200 * 1024, -1, "ntt: pass of 2^%u does not fit a CTA", a.logm);
-    B200_CUDA(cudaFuncSetAttribute(k_ntt_pass2, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));     // per device, idempotent
+    auto kern = a.pre.mode == NTT_SCALE_GEOMETRIC ? k_ntt_pass2<true> : k_ntt_pass2<false>;
+    B200_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));     // per device, idempotent
     dim3 grid((unsigned)(lines >> a.log_g), (unsigned)batch);
-    k_ntt_pass2<<<grid, threads, smem, st>>>(a);
+    kern<<<grid, threads, smem, st>>>(a);
     B200_CUDA(cudaGetLastError());
     return 0;
 }
@@ -379,9 +402,10 @@ static int launch_pass_v1(PassArgs& a, uint64_t lines, int batch, cudaStream_t s
     const uint32_t nbf = (1u << (a.logm + log_g)) >> 1;
     uint32_t threads = nbf < 32 ? 32 : (nbf > 1024 ? 1024 : nbf);
     if (cfg.ntt_threads >= 32 && cfg.ntt_threads <= 1024 && (uint32_t)cfg.ntt_threads < threads) threads = (uint32_t)cfg.ntt_threads;
-    B200_CUDA(cudaFuncSetAttribute(k_ntt_pass, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));     // per device, idempotent
+    auto kern = a.pre.mode == NTT_SCALE_GEOMETRIC ? k_ntt_pass<true> : k_ntt_pass<false>;
+    B200_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));     // per device, idempotent
     dim3 grid((unsigned)(lines >> log_g), (unsigned)batch);
-    k_ntt_pass<<<grid, threads, smem, st>>>(a);
+    kern<<<grid, threads, smem, st>>>(a);
     B200_CUDA(cudaGetLastError());
     return 0;
 }
@@ -434,6 +458,8 @@ int ntt_run(NttPlan* p, const Fr* d_src, size_t src_stride, size_t n_in, Fr* d_t
     const uint64_t N = 1ull << log_n;
     B200_CHECK(n_in <= N, -1, "ntt: n_in %zu > N", n_in);
     B200_CHECK(p && p->log_n == log_n && fp_eq(p->omega, omega), -1, "ntt: plan does not match (log_n, omega)");
+    B200_CHECK(post.mode != NTT_SCALE_GEOMETRIC && (pre.mode != NTT_SCALE_GEOMETRIC || (pre.lo && pre.hi && pre.lo_bits <= log_n)), -1,
+               "ntt: the geometric scale is a pre-scale with both power tables");
     ProfScope ps(PROF_NTT, st);
     PassArgs a;
     memset(&a, 0, sizeof a);
@@ -462,6 +488,7 @@ int ntt_run_sharded(NttPlan* const* plans, int ndev, const int* dev_ids, const F
     B200_CHECK(log_n >= 12 && log_n <= 28, -1, "sharded ntt: log_n = %u out of range [12, 28]", log_n);
     const uint64_t N = 1ull << log_n;
     B200_CHECK(n_in <= N, -1, "sharded ntt: n_in > N");
+    B200_CHECK(pre.mode != NTT_SCALE_GEOMETRIC && post.mode != NTT_SCALE_GEOMETRIC, -1, "sharded ntt: the geometric pre-scale is not supported");
     for (int g = 0; g < ndev; ++g) B200_CHECK(plans[g] && plans[g]->log_n == log_n && fp_eq(plans[g]->omega, omega), -1, "sharded ntt: plan %d does not match", g);
     int cur = 0;
     cudaGetDevice(&cur);
@@ -479,8 +506,8 @@ int ntt_run_sharded(NttPlan* const* plans, int ndev, const int* dev_ids, const F
             a.peer_on = 1; a.log_slice = log_n - log_d; a.block0 = (uint32_t)(blocks / ndev * g);
             for (int h = 0; h < ndev; ++h) { a.src_peers[h] = bufs_r[r.in_buf][h]; a.dst_peers[h] = const_cast<Fr*>(bufs_r[r.out_buf][h]); }
             B200_CUDA(cudaSetDevice(dev_ids[g]));
-            B200_CUDA(cudaFuncSetAttribute(k_ntt_pass2, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-            k_ntt_pass2<<<dim3((unsigned)(blocks / ndev), 1), threads, smem, st[g]>>>(a);
+            B200_CUDA(cudaFuncSetAttribute(k_ntt_pass2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            k_ntt_pass2<false><<<dim3((unsigned)(blocks / ndev), 1), threads, smem, st[g]>>>(a);
             B200_CUDA(cudaGetLastError());
             B200_CUDA(cudaEventRecord(ev[g], st[g]));
         }

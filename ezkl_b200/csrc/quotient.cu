@@ -18,9 +18,13 @@ namespace b200 {
 
 struct QLoadDev { const Fr* col; uint32_t offset, pad; };      // 16 B: column pointer resolved on the host
 
-template <int NSLOT>
+// PARTS: one coset part of the extended domain (quotient_eval_part_run).  Row idx < 2^k of part r loads column element
+// ((idx + offset) & mask) << pad, where pad = 0 for a part column and log2 d for a full extended column whose pointer is already
+// advanced by r, and stores its result at out[idx << out_shift] with out advanced by r.  A separate instantiation: the
+// whole-domain kernels keep their code.
+template <int NSLOT, bool PARTS>
 __global__ void __launch_bounds__(128) k_quotient_eval(const uint4* __restrict__ blob, uint32_t blob_u4, uint32_t o_loads_u4, uint32_t o_consts_u4, uint32_t mask,
-                                                        uint32_t n_instr, Fr* __restrict__ out) {
+                                                        uint32_t n_instr, Fr* __restrict__ out, uint32_t out_shift) {
     extern __shared__ uint4 sh[];
     for (uint32_t i = threadIdx.x; i < blob_u4; i += blockDim.x) sh[i] = blob[i];
     __syncthreads();
@@ -37,7 +41,8 @@ __global__ void __launch_bounds__(128) k_quotient_eval(const uint4* __restrict__
         if (k == QSRC_SLOT) return slots[i & (NSLOT - 1)];
         if (k == QSRC_CONST) return fp_load(consts + i);
         const QLoadDev l = loads[i];
-        return fp_load(l.col + ((idx + l.offset) & mask));
+        if constexpr (PARTS) return fp_load(l.col + (((idx + l.offset) & mask) << l.pad));
+        else return fp_load(l.col + ((idx + l.offset) & mask));
     };
 #pragma unroll 1
     for (uint32_t pc = 0; pc < n_instr; ++pc) {
@@ -58,14 +63,19 @@ __global__ void __launch_bounds__(128) k_quotient_eval(const uint4* __restrict__
         if (!(in.op_dst & Q_NOSTORE)) slots[(in.op_dst >> 8) & (NSLOT - 1)] = r;
         prev = r;
     }
-    fp_store(out + idx, prev);           // the row's result is the last instruction's (zero for an empty program)
+    // the row's result is the last instruction's (zero for an empty program)
+    if constexpr (PARTS) fp_store(out + ((size_t)idx << out_shift), prev);
+    else fp_store(out + idx, prev);
 }
 
-int quotient_eval_run(const Fr* const* h_col_ptrs, size_t n_cols, uint32_t ext_k, const QLoad* h_loads, size_t n_loads, const Fr* h_consts, size_t n_consts,
-                      const QInstr* h_prog, size_t n_instr, Fr* d_out, QuotientWorkspace& ws, cudaStream_t st) {
-    B200_CHECK(ext_k >= 1 && ext_k <= 28, -1, "quotient_eval: ext_k %u out of range", ext_k);
+// shared by both entry points: validates the program against n_cols columns and a row domain of 2^log_rows, stages it, launches.
+// col_shift == nullptr: the whole extended domain (offsets < 2^log_rows); otherwise one coset part (out_shift = log2 d).
+static int quotient_launch(const Fr* const* h_col_ptrs, const uint32_t* col_shift, size_t n_cols, uint32_t log_rows, const QLoad* h_loads, size_t n_loads,
+                           const Fr* h_consts, size_t n_consts, const QInstr* h_prog, size_t n_instr, Fr* d_out, uint32_t out_shift, QuotientWorkspace& ws,
+                           cudaStream_t st) {
+    B200_CHECK(log_rows >= 1 && log_rows <= 28, -1, "quotient_eval: ext_k %u out of range", log_rows);
     B200_CHECK(n_instr < (1u << 24) && n_loads < (1u << 30) && n_consts < (1u << 30), -1, "quotient_eval: program too large");
-    const uint32_t N = 1u << ext_k;
+    const uint32_t N = 1u << log_rows;
     // validate the program on the host so the kernel can index without checks
     for (size_t i = 0; i < n_loads; ++i) B200_CHECK(h_loads[i].column < n_cols && h_loads[i].offset < N, -1, "quotient_eval: load %zu out of range", i);
     uint32_t max_slot = 0;
@@ -88,7 +98,7 @@ int quotient_eval_run(const Fr* const* h_col_ptrs, size_t n_cols, uint32_t ext_k
     std::vector<uint8_t> blob(total, 0);
     if (n_instr) memcpy(blob.data(), h_prog, sizeof(QInstr) * n_instr);
     for (size_t i = 0; i < n_loads; ++i) {
-        QLoadDev l; l.col = h_col_ptrs[h_loads[i].column]; l.offset = h_loads[i].offset; l.pad = 0;
+        QLoadDev l; l.col = h_col_ptrs[h_loads[i].column]; l.offset = h_loads[i].offset; l.pad = col_shift ? col_shift[h_loads[i].column] : 0;
         memcpy(blob.data() + o_loads + sizeof(QLoadDev) * i, &l, sizeof l);
     }
     if (n_consts) memcpy(blob.data() + o_consts, h_consts, sizeof(Fr) * n_consts);
@@ -103,19 +113,39 @@ int quotient_eval_run(const Fr* const* h_col_ptrs, size_t n_cols, uint32_t ext_k
     const size_t smem = (size_t)blob_u4 * 16;
     const dim3 grid(div_up(N, 128));
     ProfScope ps(PROF_QUOTIENT, st);
-#define B200_QLAUNCH(NS)                                                                                                              \
+#define B200_QLAUNCH(NS, PARTS)                                                                                                       \
     do {                                                                                                                              \
-        B200_CUDA(cudaFuncSetAttribute(k_quotient_eval<NS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024 + 64));            \
-        k_quotient_eval<NS><<<grid, 128, smem, st>>>(reinterpret_cast<const uint4*>(d), blob_u4, (uint32_t)(o_loads / 16), (uint32_t)(o_consts / 16), N - 1, \
-                                                     (uint32_t)n_instr, d_out);                                                        \
+        B200_CUDA(cudaFuncSetAttribute(k_quotient_eval<NS, PARTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024 + 64));     \
+        k_quotient_eval<NS, PARTS><<<grid, 128, smem, st>>>(reinterpret_cast<const uint4*>(d), blob_u4, (uint32_t)(o_loads / 16), (uint32_t)(o_consts / 16), \
+                                                            N - 1, (uint32_t)n_instr, d_out, out_shift);                                \
     } while (0)
-    if (max_slot < 32) B200_QLAUNCH(32);
-    else if (max_slot < 64) B200_QLAUNCH(64);
-    else if (max_slot < 128) B200_QLAUNCH(128);
-    else B200_QLAUNCH(256);
+    if (col_shift) {
+        if (max_slot < 32) B200_QLAUNCH(32, true);
+        else if (max_slot < 64) B200_QLAUNCH(64, true);
+        else if (max_slot < 128) B200_QLAUNCH(128, true);
+        else B200_QLAUNCH(256, true);
+    } else {
+        if (max_slot < 32) B200_QLAUNCH(32, false);
+        else if (max_slot < 64) B200_QLAUNCH(64, false);
+        else if (max_slot < 128) B200_QLAUNCH(128, false);
+        else B200_QLAUNCH(256, false);
+    }
 #undef B200_QLAUNCH
     B200_CUDA(cudaGetLastError());
     return 0;
+}
+
+int quotient_eval_run(const Fr* const* h_col_ptrs, size_t n_cols, uint32_t ext_k, const QLoad* h_loads, size_t n_loads, const Fr* h_consts, size_t n_consts,
+                      const QInstr* h_prog, size_t n_instr, Fr* d_out, QuotientWorkspace& ws, cudaStream_t st) {
+    return quotient_launch(h_col_ptrs, nullptr, n_cols, ext_k, h_loads, n_loads, h_consts, n_consts, h_prog, n_instr, d_out, 0, ws, st);
+}
+
+int quotient_eval_part_run(const Fr* const* h_col_ptrs, const uint32_t* h_col_shift, size_t n_cols, uint32_t k, uint32_t log_d, const QLoad* h_loads, size_t n_loads,
+                           const Fr* h_consts, size_t n_consts, const QInstr* h_prog, size_t n_instr, Fr* d_out, QuotientWorkspace& ws, cudaStream_t st) {
+    B200_CHECK(h_col_shift || n_cols == 0, -1, "quotient_eval: part layout missing");
+    for (size_t i = 0; i < n_cols; ++i) B200_CHECK(h_col_shift[i] == 0 || h_col_shift[i] == log_d, -1, "quotient_eval: column %zu: bad part stride", i);
+    static const uint32_t no_cols = 0;
+    return quotient_launch(h_col_ptrs, n_cols ? h_col_shift : &no_cols, n_cols, k, h_loads, n_loads, h_consts, n_consts, h_prog, n_instr, d_out, log_d, ws, st);
 }
 
 }  // namespace b200

@@ -19,5 +19,10 @@ struct QuotientWorkspace { DevBuf prog; StagingRing ring; };
 // out[idx] = program(columns[c][(idx + offset) mod N], constants) for idx < N = 2^ext_k.  h_* are host arrays.
 int quotient_eval_run(const Fr* const* h_col_ptrs /*device addresses*/, size_t n_cols, uint32_t ext_k, const QLoad* h_loads, size_t n_loads,
                       const Fr* h_consts, size_t n_consts, const QInstr* h_prog, size_t n_instr, Fr* d_out, QuotientWorkspace& ws, cudaStream_t st);
+// One coset part r of the extended domain (d = 2^log_d parts of 2^k rows each): out[idx << log_d] = program(...) for idx < 2^k, where
+// column c is read at ((idx + offset) mod 2^k) << h_col_shift[c].  h_col_shift[c] = 0: a part column (2^k values of that part);
+// log_d: a full extended column whose device address is already advanced by r.  d_out is advanced by r.  Offsets are Rotation(rot) mod 2^k.
+int quotient_eval_part_run(const Fr* const* h_col_ptrs, const uint32_t* h_col_shift, size_t n_cols, uint32_t k, uint32_t log_d, const QLoad* h_loads, size_t n_loads,
+                           const Fr* h_consts, size_t n_consts, const QInstr* h_prog, size_t n_instr, Fr* d_out, QuotientWorkspace& ws, cudaStream_t st);
 
 }  // namespace b200

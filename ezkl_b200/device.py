@@ -158,6 +158,27 @@ def ntt(src: torch.Tensor, log_n: int, omega, *, n_in: int | None = None, pre=No
     return out
 
 
+def coeff_to_extended_part(src: torch.Tensor, domain, part: int, *, out: torch.Tensor | None = None, tmp: torch.Tensor | None = None) -> torch.Tensor:
+    """src [batch, n_coeffs, 4] (n_coeffs <= n) -> out [batch, n, 4]: part `part` of every polynomial's extended coset,
+    coeff_to_extended(p)[part::d] (b200_coeff_to_extended_part_dev).  domain: a halo2.EvaluationDomain."""
+    if src.dim() == 2:
+        src = src.unsqueeze(0)
+    _chk(src, 4)
+    batch, n_src = src.shape[0], src.shape[1]
+    n = 1 << domain.k
+    if out is None:
+        out = torch.empty((batch, n, 4), dtype=torch.int64, device="cuda")
+    if tmp is None:
+        tmp = torch.empty((batch, n, 4), dtype=torch.int64, device="cuda")
+    _chk(out, 4)
+    _chk(tmp, 4)
+    assert out.numel() >= batch * n * 4 and tmp.numel() >= batch * n * 4
+    nat.check(nat.lib().b200_coeff_to_extended_part_dev(nat.dev(src.data_ptr()), C.c_size_t(n_src), C.c_size_t(n_src), nat.dev(tmp.data_ptr()),
+                                                        nat.dev(out.data_ptr()), C.c_size_t(n), C.c_uint32(domain.k), C.c_uint32(domain.extended_k),
+                                                        C.c_uint32(part), nat.ptr(domain.extended_omega), nat.ptr(domain.g_coset), C.c_size_t(batch), _stream()))
+    return out
+
+
 _OPS = {"add": 0, "sub": 1, "mul": 2, "scale": 3, "axpy": 4}
 
 

@@ -307,6 +307,49 @@ def evaluate_h_from_polys(program: QuotientProgram, polys, domain, finish: bool 
     return out
 
 
+def _parts_args(program: QuotientProgram, lengths, domain, finish: bool):
+    """Arguments shared by b200_evaluate_h_parts and its device form, after the column pointers (include/ezkl_b200_parts.h)."""
+    lens = (C.c_size_t * max(1, len(lengths)))(*lengths)
+    loads, consts, prog = program.arrays()
+    t = domain.t_evaluations
+    keep = (loads, consts, prog)
+    args = [lens, C.c_size_t(len(lengths)), C.c_uint32(domain.k), C.c_uint32(domain.extended_k), nat.ptr(domain.extended_omega), nat.ptr(domain.g_coset),
+            loads.ctypes.data_as(C.c_void_p), C.c_size_t(loads.shape[0]), nat.ptr(consts) if consts.size else None, C.c_size_t(consts.shape[0]),
+            prog.ctypes.data_as(C.c_void_p), C.c_size_t(prog.shape[0]), nat.ptr(t) if finish else None, C.c_uint32(t.shape[0] if finish else 0),
+            nat.ptr(domain.extended_omega_inv) if finish else None, nat.ptr(domain.extended_ifft_divisor) if finish else None]
+    return args, keep
+
+
+def evaluate_h_parts(program: QuotientProgram, polys, domain, finish: bool = False) -> np.ndarray:
+    """b200_evaluate_h_parts: what evaluate_h_from_polys computes, byte for byte, evaluated one coset part of the extended domain at a time,
+    so that no column's full coset is ever on the device.  Columns are coefficient form (len <= n) or on the extended domain
+    (len == 2^extended_k); finish=True returns the quotient's coefficients (all 2^extended_k of them)."""
+    nat.ensure_init()
+    cols = [nat.as_u64(c, 4) for c in polys]
+    N = 1 << domain.extended_k
+    args, _keep = _parts_args(program, [c.shape[0] for c in cols], domain, finish)
+    out = np.zeros((N, 4), np.uint64)
+    nat.check(nat.lib().b200_evaluate_h_parts(nat.ptr_array(cols) if cols else None, *args, nat.ptr(out)))
+    return out
+
+
+def evaluate_h_parts_device(program: QuotientProgram, columns, domain, finish: bool = False, out=None):
+    """Device form of evaluate_h_parts: columns = list of torch int64 CUDA tensors [len, 4] (len <= n: coefficients, len == 2^extended_k:
+    extended values, read in place); enqueued on torch's current stream.  Returns out [2^extended_k, 4]."""
+    import torch
+    from .device import _stream
+    N = 1 << domain.extended_k
+    for c in columns:
+        assert c.is_cuda and c.dtype == torch.int64 and c.is_contiguous() and c.dim() == 2 and c.shape[1] == 4
+    if out is None:
+        out = torch.empty((N, 4), dtype=torch.int64, device="cuda")
+    assert out.is_cuda and out.dtype == torch.int64 and out.is_contiguous() and out.shape == (N, 4)
+    args, _keep = _parts_args(program, [c.shape[0] for c in columns], domain, finish)
+    ptrs = (C.c_void_p * max(1, len(columns)))(*[c.data_ptr() for c in columns])
+    nat.check(nat.lib().b200_evaluate_h_parts_dev(ptrs, *args, nat.dev(out.data_ptr()), _stream()))
+    return out
+
+
 def evaluate_h_device(program: QuotientProgram, columns, k: int, ext_k: int, out=None):
     """Device path: columns = list of torch int64 CUDA tensors [2^ext_k, 4]; enqueued on torch's current stream."""
     import torch

@@ -228,6 +228,23 @@ class EvaluationDomain:
                                                               nat.ptr(self.extended_omega), nat.ptr(self.g_coset), nat.ptr_array(outs)))
         return outs
 
+    def coeff_to_extended_part(self, a, part: int) -> np.ndarray:
+        """Part `part` of coeff_to_extended(a): its values at zeta * extended_omega^part * omega^t, t < n, i.e. coeff_to_extended(a)[part::d]
+        with d = 2^(extended_k - k).  a has at most n coefficients (include/ezkl_b200_parts.h)."""
+        return self.coeff_to_extended_part_batch([a], part)[0]
+
+    def coeff_to_extended_part_batch(self, cols, part: int):
+        cols = [_fr(c) for c in cols]
+        outs = [np.zeros((self.n, 4), np.uint64) for _ in cols]
+        if cols:
+            n_coeffs = cols[0].shape[0]
+            if any(c.shape[0] != n_coeffs for c in cols) or n_coeffs > self.n:
+                raise nat.B200Error("coeff_to_extended_part: polynomials need one length <= n = %d" % self.n)
+            nat.check(nat.lib().b200_coeff_to_extended_part_batch(nat.ptr_array(cols), C.c_size_t(len(cols)), C.c_size_t(n_coeffs), C.c_uint32(self.k),
+                                                                   C.c_uint32(self.extended_k), C.c_uint32(part), nat.ptr(self.extended_omega),
+                                                                   nat.ptr(self.g_coset), nat.ptr_array(outs)))
+        return outs
+
     def extended_to_coeff(self, a) -> np.ndarray:
         """Returns n * quotient_poly_degree coefficients (upstream truncates the same way)."""
         a = _fr(a).copy()
@@ -246,17 +263,28 @@ class EvaluationDomain:
         """l0, l_last, l_active_row on the extended coset, as halo2 keygen_pk builds them (UPSTREAM plonk/keygen.rs; entered
         from /root/reference/src/pfsys/mod.rs:396): l0 = L_0, l_last = L_{n - blinding_factors - 1},
         l_active_row = 1 - (l_last + l_blind) with l_blind = sum of the Lagrange polynomials of the last blinding rows."""
+        l0, l_last, l_blind = self.coeff_to_extended_batch(self._l_basis_coeffs(blinding_factors))
+        ones = np.tile(F.fr_to_limbs(1), (self.extended_len(), 1))
+        l_active = poly_op("sub", ones, poly_op("add", l_last, l_blind))
+        return l0, l_last, l_active
+
+    def keygen_l_coeffs(self, blinding_factors: int):
+        """l0, l_last, l_active_row of keygen_l_polys in coefficient form (n coefficients each); their cosets are exactly keygen_l_polys'
+        (l_active_row = 1 - (l_last + l_blind) holds coefficient-wise, the constant 1 being the coefficient vector [1, 0, ...])."""
+        l0, l_last, l_blind = self._l_basis_coeffs(blinding_factors)
+        unit = np.zeros((self.n, 4), np.uint64)
+        unit[0] = F.fr_to_limbs(1)
+        return l0, l_last, poly_op("sub", unit, poly_op("add", l_last, l_blind))
+
+    def _l_basis_coeffs(self, blinding_factors: int):
+        """Coefficients of L_0, L_{n - blinding_factors - 1} and the sum of the last blinding rows' Lagrange polynomials."""
         n = self.n
         one = F.fr_to_limbs(1)
         rows = np.zeros((3, n, 4), np.uint64)
         rows[0, 0] = one
         rows[1, n - blinding_factors - 1] = one
         rows[2, n - blinding_factors:] = one
-        coeffs = self.lagrange_to_coeff_batch([rows[0], rows[1], rows[2]])
-        l0, l_last, l_blind = self.coeff_to_extended_batch(coeffs)
-        ones = np.tile(one, (self.extended_len(), 1))
-        l_active = poly_op("sub", ones, poly_op("add", l_last, l_blind))
-        return l0, l_last, l_active
+        return self.lagrange_to_coeff_batch([rows[0], rows[1], rows[2]])
 
     def rotate_omega(self, value: int, rotation: int) -> int:
         r = F.FR_MODULUS

@@ -174,8 +174,16 @@ class Keys:
         self.l0, self.l_last, self.l_active = self.domain.keygen_l_polys(cs.blinding_factors)
         x_coeff = np.zeros((n, 4), np.uint64)
         x_coeff[1] = F.fr_to_limbs(1)
+        self.x_poly = x_coeff
         self.x_coset = self.domain.coeff_to_extended(x_coeff)
         self.vk_repr = vk_repr % R          # UNPINNED: upstream hashes the pinned verifying key (Blake2b of its debug string) into this scalar
+        self._l_coeffs = None
+
+    def l_polys(self):
+        """(l0, l_last, l_active) in coefficient form, derived on first use: what the per-part quotient reads instead of their cosets."""
+        if self._l_coeffs is None:
+            self._l_coeffs = self.domain.keygen_l_coeffs(self.cs.blinding_factors)
+        return self._l_coeffs
 
 
 def sigma_labels(k: int, num_columns: int, cycles_next: dict) -> list:
@@ -205,9 +213,14 @@ def _ints(col_wire) -> list:
 
 
 # ---- the prover ---------------------------------------------------------------------------------------------------------------------
-def create_proof(keys: Keys, advice, instances=(), rng=None, trace=None) -> bytes:
+def create_proof(keys: Keys, advice, instances=(), rng=None, trace=None, quotient: str = "full") -> bytes:
     """advice: list of num_advice columns (python ints; rows >= n - blinding_factors are overwritten with blinding values).
-    Returns the proof bytes (EvmTranscript stream).  `trace`, if a dict, receives the challenges and intermediate columns."""
+    Returns the proof bytes (EvmTranscript stream).  `trace`, if a dict, receives the challenges and intermediate columns.
+    quotient: "full" evaluates h over the whole extended domain at once (the key's cosets as columns); "parts" evaluates it one
+    coset part at a time from coefficient-form columns only (evaluation.evaluate_h_parts): the same bytes, with device memory
+    of about one part per column instead of one coset per column."""
+    if quotient not in ("full", "parts"):
+        raise ValueError("create_proof: quotient must be 'full' or 'parts', not %r" % (quotient,))
     cs, params, dom = keys.cs, keys.params, keys.domain
     n, k, bf = params.n, params.k, cs.blinding_factors
     u = n - bf - 1
@@ -292,8 +305,16 @@ def create_proof(keys: Keys, advice, instances=(), rng=None, trace=None) -> byte
     for i, (mc, pc) in enumerate(L["lookup"]):
         columns[mc], columns[pc] = lk_polys[i]
     columns[L["l0"]], columns[L["l_last"]], columns[L["l_active"]], columns[L["x"]] = keys.l0, keys.l_last, keys.l_active, keys.x_coset
+    if quotient == "parts":                # the key's columns in coefficient form too: nothing of 2^ext_k elements reaches the device but the output
+        for i in range(cs.num_fixed):
+            columns[na + i] = keys.fixed_polys[i]
+        for i, c in enumerate(L["sigma"]):
+            columns[c] = keys.sigma_polys[i]
+        columns[L["l0"]], columns[L["l_last"]], columns[L["l_active"]] = keys.l_polys()
+        columns[L["x"]] = keys.x_poly
     prog = ev.QuotientProgram(cs.numerator(beta, gamma, y))
-    h = ev.evaluate_h_from_polys(prog, columns, dom, finish=True)[: n * dom.quotient_poly_degree]
+    evaluate = ev.evaluate_h_parts if quotient == "parts" else ev.evaluate_h_from_polys
+    h = evaluate(prog, columns, dom, finish=True)[: n * dom.quotient_poly_degree]
     pieces = [np.ascontiguousarray(h[i * n:(i + 1) * n]) for i in range(dom.quotient_poly_degree)]
     for c in params.commit_batch(pieces):
         tr.write_ec_point(c)
